@@ -4,6 +4,7 @@ greedy decode).
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one rank per GPU under torchrun)
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle) on the host cores
+  python bench.py ... --dump-outputs DIR                   # also write what the last timed step returned to DIR/<name>.npy
 
 One "step" = one GromaModel.generate() over a batch of 16 synthetic 448x448 images + 512-token prompts per GPU
 (BASELINE.json configs[3]; weak scaling = configs[4]), random-init Groma-7B weights (no network for checkpoints).
@@ -42,10 +43,52 @@ def parse_args():
     ap.add_argument("--profile", action="store_true", help="print a per-stage CUDA-event breakdown of one step to stderr")
     ap.add_argument("--ncu-range", action="store_true",
                     help="wrap ONE extra step in cudaProfilerStart/Stop (use with ncu --profile-from-start off --graph-profiling node)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what generate() returned in the last one to DIR/<name>.npy (float32 / "
+                         "float64; outputs larger than 2^21 elements as a fixed seeded sample), for comparing two builds")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 METRIC = "images/sec Groma-7B 448px prefill+128-tok decode"
+
+
+DUMP_SAMPLE = 1 << 21          # elements kept of an output larger than this (8 MB in float32)
+
+
+def _dump_sample(t: torch.Tensor, n: int, seed: int) -> torch.Tensor:
+    """`t` whole if it has at most `n` elements, else `n` of its elements at flat indices drawn from `seed` (sorted): the same
+    indices for the same shape, so two runs compare element for element."""
+    if t.numel() <= n:
+        return t
+    idx = torch.randint(t.numel(), (n,), generator=torch.Generator().manual_seed(seed)).sort().values.to(t.device)
+    return t[torch.unravel_index(idx, t.shape)]
+
+
+def dump_outputs(out_dir: str, seq: torch.Tensor, out) -> dict:
+    """What GromaModel.generate() returned to its caller: the sequences (token ids, exact in float64), the selected boxes of
+    every image, the image and region features and the KV cache.  Returns {name: bytes written}."""
+    import numpy as np
+    vis = out.hidden_states[0][-1]
+    kv = [t for layer in out.past_key_values for t in layer]          # 2 x layers tensors [B, heads, ctx, head_dim]
+    arrays = {
+        "sequences": seq.double(),
+        "pred_boxes": torch.cat(vis["pred_boxes"]).float(),
+        "regions_per_image": torch.tensor([len(b) for b in vis["pred_boxes"]], dtype=torch.float64),
+        "image_features": _dump_sample(vis["image_features"], DUMP_SAMPLE, 1).float(),
+        "region_features": _dump_sample(vis["region_features"], DUMP_SAMPLE, 2).float(),
+        "past_key_values": torch.stack([_dump_sample(t, DUMP_SAMPLE // len(kv), 3 + i) for i, t in enumerate(kv)]).float(),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    written = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        written[name] = a.nbytes
+    assert sum(written.values()) <= 64 << 20, written
+    return written
 
 
 def make_inputs(cfg, B, T_text, seed, tok):
@@ -214,6 +257,7 @@ def main():
             seq = seq.cpu()
         realised["R"] = [len(b) for b in boxes]
         realised["T"] = model._path_cfg.grid ** 2 // 4 + args.prompt - 2 + 2 * max(realised["R"])
+        realised["outputs"] = (seq, out)
         return seq
 
     def barrier():
@@ -261,6 +305,10 @@ def main():
     ms_dev, launches_dev = timed(False, args.steps)
     ms_e2e, _ = timed(True, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    dumped = None
+    if args.dump_outputs and rank == 0:     # before the roofline below, which overwrites the KV cache
+        dumped = dump_outputs(args.dump_outputs, *realised.pop("outputs"))
+    realised.pop("outputs", None)
 
     # kernels launched inside one timed step: C-ABI launches made eagerly + kernels replayed from the decode graph
     graph_kernels = getattr(model, "_graph_kernels", 0)
@@ -288,6 +336,8 @@ def main():
                     "h2d_bytes_per_step": int(images_h.numel() * 4 + ids_h.numel() * 8),
                     "d2h_bytes_per_step": int(B * world * (args.prompt + args.new) * 8)},
             "gpu_launches": int(gpu_launches), "roofline": roof}
+    if dumped is not None:
+        line["dumped_outputs"] = {"dir": args.dump_outputs, "bytes": dumped}
     if sd_for_cpu is not None:
         sd_cpu = {k: v.float().cpu() for k, v in sd_for_cpu.items()}
         del sd_for_cpu

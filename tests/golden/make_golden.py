@@ -2,8 +2,14 @@
 2-image batch.  The reference itself cannot be imported in this image (SURVEY.md T12), so these vectors pin the
 restatement against silent drift -- and the GPU path (tests/test_golden_gpu.py) against the restatement -- rather
 than against the reference.   python -m tests.golden.make_golden
+
+The oracle runs under CANONICAL_CPU_ENV so that the fixture is bit-for-bit what any x86-64 machine computes: with the
+default settings the fp32 sums differ with the CPU's vector ISA and thread count, and the bf16 rounding points turn such
+last-bit differences into different greedy tokens or NMS orders wherever two candidates are nearly tied.
 """
 import os
+import subprocess
+import sys
 
 import torch
 
@@ -12,6 +18,10 @@ from oracle.groma_oracle import Oracle
 from oracle.weights import make_state_dict
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+# one thread, ATen's portable (non-AVX) kernels, oneDNN at its baseline ISA, MKL in conditional-numerical-reproducibility
+# mode; all are read when torch loads, hence the child process of run_canonical()
+CANONICAL_CPU_ENV = {"ATEN_CPU_CAPABILITY": "default", "ONEDNN_MAX_CPU_ISA": "SSE41", "MKL_CBWR": "COMPATIBLE",
+                     "OMP_NUM_THREADS": "1", "MKL_NUM_THREADS": "1"}
 
 
 def inputs():
@@ -37,7 +47,18 @@ def run_oracle():
                 last_logits=out["logits"][:, -1].clone(), step_logits=out["step_logits"], topk=o.stages["topk"].clone())
 
 
+def run_canonical(path):
+    """run_oracle() in a child process under CANONICAL_CPU_ENV; its outputs are saved to `path` and returned."""
+    root = os.path.dirname(os.path.dirname(HERE))
+    subprocess.run([sys.executable, "-m", "tests.golden.make_golden", path], cwd=root, env=dict(os.environ, **CANONICAL_CPU_ENV),
+                   check=True)
+    return torch.load(path)
+
+
 if __name__ == "__main__":
-    out = run_oracle()
-    torch.save(out, os.path.join(HERE, "tiny_forward.pt"))
-    print({k: (tuple(v.shape) if hasattr(v, "shape") else len(v)) for k, v in out.items()})
+    if len(sys.argv) > 1:           # the child of run_canonical()
+        assert all(os.environ.get(k) == v for k, v in CANONICAL_CPU_ENV.items())
+        torch.save(run_oracle(), sys.argv[1])
+    else:
+        out = run_canonical(os.path.join(HERE, "tiny_forward.pt"))
+        print({k: (tuple(v.shape) if hasattr(v, "shape") else len(v)) for k, v in out.items()})

@@ -51,3 +51,34 @@ def test_reference_arm_line():
     assert d["impl"] == "reference" and d["unit"] == "images/sec" and d["value"] > 0
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0 and d["e2e"]["value"] == d["value"]
     assert d["cpu_baseline"]["value"] == d["value"] and d["cpu_baseline"]["kind"] in ("port", "reference")
+
+
+def test_dump_outputs_writes_what_generate_returned(tmp_path):
+    """bench.py --dump-outputs: float32 / float64 arrays, token ids exact, large outputs as the same seeded sample every run,
+    64 MB at most -- on the full-size shapes of a generate() result (KV cache shortened to 300 positions of 320)."""
+    from types import SimpleNamespace
+
+    import numpy as np
+    import torch
+
+    import bench
+    g = torch.Generator().manual_seed(0)
+    B, R, H = 16, 100, 4096
+    boxes = [torch.rand(R, 4, generator=g) for _ in range(B)]
+    vis = {"pred_boxes": boxes, "image_features": torch.randn(B, 256, H, generator=g).bfloat16(),
+           "region_features": torch.randn(B * R, H, generator=g).bfloat16()}
+    kv_store = torch.randn(32, 2, 2, 32, 320, 128, generator=g).bfloat16()
+    out = SimpleNamespace(hidden_states=((None, vis),), past_key_values=tuple((kv_store[i, 0, :, :, :300], kv_store[i, 1, :, :, :300])
+                                                                              for i in range(32)))
+    seq = torch.randint(0, 32003, (B, 640), generator=g)
+    written = bench.dump_outputs(str(tmp_path / "a"), seq, out)
+    bench.dump_outputs(str(tmp_path / "b"), seq, out)
+    assert sum(written.values()) <= 64 << 20
+    for name in written:
+        a, b = np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy")
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b), name
+    assert np.array_equal(np.load(tmp_path / "a" / "sequences.npy").astype(np.int64), seq.numpy())
+    assert np.array_equal(np.load(tmp_path / "a" / "pred_boxes.npy"), torch.cat(boxes).numpy())
+    img = np.load(tmp_path / "a" / "image_features.npy")
+    assert img.shape == (bench.DUMP_SAMPLE,) and np.isin(img, vis["image_features"].float().numpy()).all()
+    assert np.load(tmp_path / "a" / "past_key_values.npy").shape == (64, bench.DUMP_SAMPLE // 64)

@@ -1,6 +1,9 @@
 """Drop-in boundary, host side (SURVEY.md section 8b): every name the reference's eval scripts import from the `groma` package
 exists in this repo's `groma` package, the scripts' module bodies execute on top of it, `model.generation_config` carries the
-checkpoint's EOS / pad ids, and `AutoModel.from_pretrained` resolves to GromaModel.  No GPU needed."""
+checkpoint's EOS / pad ids, and `AutoModel.from_pretrained` resolves to GromaModel.  No GPU needed.
+
+What the scripts' module bodies execute -- their import statements and the base classes of the classes they define -- is
+stored in tests/golden/eval_script_imports.json (tests/golden/make_eval_imports_golden.py)."""
 import ast
 import importlib
 import json
@@ -11,23 +14,28 @@ import types
 import pytest
 import torch
 
-REF_EVAL = "/root/reference/groma/eval"
 SCRIPTS = ["run_groma.py", "run_ddetr.py", "eval_rec.py", "eval_lvis.py", "model_vg.py", "model_refcocog.py", "model_vqa.py"]
 # modules of the reference's `groma` package that are on the path and therefore provided by this repo
 PROVIDED = {"groma.utils", "groma.constants", "groma.model.groma", "groma.model.ddetr", "groma.data.conversation"}
+with open(os.path.join(os.path.dirname(__file__), "golden", "eval_script_imports.json")) as _f:
+    EVAL_SCRIPTS = json.load(_f)
 
 
-def _groma_imports(path):
-    tree = ast.parse(open(path).read())
-    for n in ast.walk(tree):
-        if isinstance(n, ast.ImportFrom) and n.module and n.module.startswith("groma"):
-            yield n.module, [a.name for a in n.names]
+def _groma_imports(script):
+    for st in EVAL_SCRIPTS[script]["imports"]:
+        if st.get("from") and st["from"].startswith("groma"):
+            yield st["from"], [n for n, _ in st["names"]]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_EVAL), reason="/root/reference not present (GPU box)")
+def _import_node(st):
+    if "import" in st:
+        return ast.Import(names=[ast.alias(name=n, asname=a) for n, a in st["import"]])
+    return ast.ImportFrom(module=st["from"], names=[ast.alias(name=n, asname=a) for n, a in st["names"]], level=st["level"])
+
+
 @pytest.mark.parametrize("script", SCRIPTS)
 def test_names_the_eval_scripts_import_exist(script):
-    for mod, names in _groma_imports(os.path.join(REF_EVAL, script)):
+    for mod, names in _groma_imports(script):
         if mod not in PROVIDED:
             assert mod.startswith("groma.data.datasets"), f"{script} imports {mod}, which is neither provided nor a dataset module"
             continue
@@ -48,15 +56,15 @@ class _Anything(types.ModuleType):
         return lambda *a, **k: None
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_EVAL), reason="/root/reference not present (GPU box)")
 @pytest.mark.parametrize("script", SCRIPTS)
 def test_eval_script_module_bodies_execute_on_this_package(script, monkeypatch):
-    """Execute the reference script's module body (imports, helper definitions; not `__main__`) with `groma.*` resolving to THIS
-    repo; only packages missing from the image (mmcv, mmdet, pycocotools, lvis) and the dataset modules are stood in for."""
-    path = os.path.join(REF_EVAL, script)
+    """Execute what the reference script's module body executes (its imports, and the base classes of the classes it defines;
+    its functions take no defaults or decorators, and `__main__` does not run) with `groma.*` resolving to THIS repo; only
+    packages missing from the image (mmcv, mmdet, pycocotools, lvis) and the dataset modules are stood in for."""
+    body = EVAL_SCRIPTS[script]
     absent_roots = {"mmcv", "mmdet", "pycocotools", "lvis"}
-    for n in ast.walk(ast.parse(open(path).read())):
-        mods = [n.module] if isinstance(n, ast.ImportFrom) and n.module else [a.name for a in n.names] if isinstance(n, ast.Import) else []
+    for st in body["imports"]:
+        mods = [n for n, _ in st["import"]] if "import" in st else [st["from"]] if st["from"] else []
         for mod in mods:
             if mod.split(".")[0] in absent_roots or mod.startswith("groma.data.datasets"):
                 parts = mod.split(".")
@@ -64,8 +72,11 @@ def test_eval_script_module_bodies_execute_on_this_package(script, monkeypatch):
                     name = ".".join(parts[:i])
                     if name not in sys.modules and not name == "groma" and not name == "groma.data":
                         monkeypatch.setitem(sys.modules, name, _Anything(name))
-    ns = {"__name__": "ref_eval_" + script[:-3], "__file__": path}
-    exec(compile(open(path).read(), path, "exec"), ns)
+    ns = {"__name__": "ref_eval_" + script[:-3]}
+    module = ast.fix_missing_locations(ast.Module(body=[_import_node(st) for st in body["imports"]], type_ignores=[]))
+    exec(compile(module, script, "exec"), ns)
+    for base in body["class_bases"]:
+        assert isinstance(eval(base, ns), type), f"{script}: base class {base} does not resolve"
     import groma.model.groma as ours
     if "GromaModel" in ns:
         assert ns["GromaModel"] is ours.GromaModel
