@@ -399,7 +399,6 @@ class GromaModel(torch.nn.Module):
                 logits = d["logits"].clone().reshape(B, 1, -1)
             else:
                 logits = eng.decode_step(B).clone().reshape(B, 1, -1)
-            eng.check_decode_status()
             eng.past = past + 1
             labels_new = None
         loss = None
@@ -465,7 +464,6 @@ class GromaModel(torch.nn.Module):
                 self._step_logits.append(d["logits"].clone())
             steps_done = s + 1
         self._mark("decode")
-        eng.check_decode_status()
         eng.past = T + steps_done - 1
         new = out_tokens[:steps_done].t().contiguous()
         if eos_t is not None:
@@ -487,7 +485,7 @@ class GromaModel(torch.nn.Module):
     def _capture(self, B: int):
         """Capture one decode step (all 32 layers + heads + argmax + position advance) into a CUDA graph."""
         eng = self.engine
-        key = (B, eng.kv.data_ptr(), eng.kv_cap, eng.rope_cos.data_ptr(), eng.use_megakernel)
+        key = (B, eng.kv.data_ptr(), eng.kv_cap, eng.rope_cos.data_ptr())
         if self._graph is not None and self._graph[0] == key:
             return self._graph[1]
         g = torch.cuda.CUDAGraph()

@@ -6,7 +6,6 @@
 #include "decode_common.cuh"
 #include "capi_common.h"
 #include <cooperative_groups.h>
-#include <cstdlib>
 
 namespace gb {
 
@@ -249,9 +248,13 @@ GROMA_API int32_t groma_attention(const void* q, int64_t q_bs, int64_t q_rs, con
 
 // ------------------------------------------------------------------------------------------------------------------
 // Decode attention (one query token per sequence): HBM-bound streaming of the K/V cache, no tensor cores.
-// One CTA per (head, batch row); 8 warps; a warp covers two keys per step (16 lanes x 16 bytes = one 256-byte K row per
-// half-warp), four steps in flight; online softmax per half-warp, merged through shared memory at the end.
 // Semantics = groma/model/groma.py:376-379 + eager LLaMA attention: every cached position < kv_len[b] is visible.
+// One 2-CTA cluster per (head, batch row), the keys split between the pair.  Per CTA one producer lane issues 1-D bulk copies
+// of DT_KEYS consecutive K rows and V rows (contiguous in the [B,H,cap,D] cache) into a DT_STAGES-deep shared-memory ring;
+// the DEC_WARPS consumer warps cover two keys per warp and step (16 lanes x 16 bytes = one 256-byte row per half-warp), fold
+// DT_UNROLL steps into each online-softmax update, and merge their half-warp states through shared memory, then the pair's
+// states through distributed shared memory.  Bytes in flight do not depend on registers/occupancy: 8 resident CTAs x 24 KB
+// per SM.
 namespace gb {
 
 #ifndef GROMA_DEC_WARPS
@@ -263,164 +266,6 @@ namespace gb {
 constexpr int DEC_WARPS = GROMA_DEC_WARPS;   // 2 warps/CTA, 2 CTAs (one cluster) per (batch, head): 2*B*H CTAs all resident in one wave
 constexpr int DEC_SPLIT = GROMA_DEC_SPLIT;                   // keys are split over the CTAs of a cluster; partials merge through DSMEM
 
-// streaming 16-byte load that does not allocate in L1 (the KV cache is read once per step)
-__device__ __forceinline__ uint4 ld_nc_u4(const __nv_bfloat16* p) {
-    uint4 r;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
-    return r;
-}
-
-template <int D, int DEC_UNROLL>
-__global__ void __cluster_dims__(DEC_SPLIT, 1, 1) __launch_bounds__(DEC_WARPS * 32) decode_attention_kernel(
-    const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ kc, const __nv_bfloat16* __restrict__ vc,
-    __nv_bfloat16* __restrict__ out, const int* __restrict__ kv_len, int H, long long cap, float scale_log2) {
-    static_assert(D == 128, "16 lanes x 8 dims");
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    // distributed-shared-memory rule: a CTA may only touch a peer's shared memory once that peer is known to be running.
-    // Arrive now, wait just before the first remote store -- the barrier latency hides behind the key loop.
-    cluster_arrive_relaxed();
-    asm volatile("griddepcontrol.wait;" ::: "memory");   // no-op unless launched with programmatic serialisation
-    namespace cg = cooperative_groups;
-    cg::cluster_group cluster = cg::this_cluster();
-    const int crank = (int)cluster.block_rank();
-    const int h = blockIdx.x / DEC_SPLIT, b = blockIdx.y;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int grp = lane >> 4, l = lane & 15;
-    const int n_all = kv_len[b];
-    const int per = (n_all + DEC_SPLIT - 1) / DEC_SPLIT;
-    const int k_begin = min(crank * per, n_all);
-    const int n = min(n_all, k_begin + per) - k_begin;   // this CTA's keys: [k_begin, k_begin + n)
-    const __nv_bfloat16* kb = kc + (((long long)b * H + h) * cap + k_begin) * D;
-    const __nv_bfloat16* vb = vc + (((long long)b * H + h) * cap + k_begin) * D;
-    float qf[8];
-    {
-        const uint4 qv = *reinterpret_cast<const uint4*>(q + ((long long)b * H + h) * D + l * 8);
-        const __nv_bfloat162* q2 = reinterpret_cast<const __nv_bfloat162*>(&qv);
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-            const float2 f = __bfloat1622float2(q2[t]);
-            qf[2 * t] = f.x * scale_log2;
-            qf[2 * t + 1] = f.y * scale_log2;
-        }
-    }
-    float m = -INFINITY, lsum = 0.f, acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    constexpr int STEP = DEC_WARPS * 2;  // keys per block step
-    // software pipeline: the K rows of the next step and the V rows of this step are requested before this step's
-    // arithmetic, so 8 x 16-byte loads per lane are in flight (HBM-bound: ~115 KB outstanding per SM)
-    uint4 kcur[DEC_UNROLL];
-    {
-        const int j0 = warp * 2 + grp;
-#pragma unroll
-        for (int u = 0; u < DEC_UNROLL; ++u) {
-            const int j = j0 + u * STEP;
-            kcur[u] = (j < n) ? ld_nc_u4(kb + (long long)j * D + l * 8) : make_uint4(0, 0, 0, 0);
-        }
-    }
-    for (int base = warp * 2; base < n; base += STEP * DEC_UNROLL) {   // warp-uniform trip count (shuffles below)
-        const int j0 = base + grp;
-        uint4 vv[DEC_UNROLL], knext[DEC_UNROLL];
-        float s[DEC_UNROLL];
-#pragma unroll
-        for (int u = 0; u < DEC_UNROLL; ++u) {
-            const int j = j0 + u * STEP;
-            vv[u] = (j < n) ? ld_nc_u4(vb + (long long)j * D + l * 8) : make_uint4(0, 0, 0, 0);
-        }
-#pragma unroll
-        for (int u = 0; u < DEC_UNROLL; ++u) {
-            const int j = j0 + (u + DEC_UNROLL) * STEP;
-            knext[u] = (j < n) ? ld_nc_u4(kb + (long long)j * D + l * 8) : make_uint4(0, 0, 0, 0);
-        }
-#pragma unroll
-        for (int u = 0; u < DEC_UNROLL; ++u) {
-            const __nv_bfloat162* k2 = reinterpret_cast<const __nv_bfloat162*>(&kcur[u]);
-            float d = 0.f;
-#pragma unroll
-            for (int t = 0; t < 4; ++t) {
-                const float2 f = __bfloat1622float2(k2[t]);
-                d += f.x * qf[2 * t] + f.y * qf[2 * t + 1];
-            }
-            d += __shfl_xor_sync(0xffffffffu, d, 8);
-            d += __shfl_xor_sync(0xffffffffu, d, 4);
-            d += __shfl_xor_sync(0xffffffffu, d, 2);
-            d += __shfl_xor_sync(0xffffffffu, d, 1);
-            s[u] = (j0 + u * STEP < n) ? d : -INFINITY;
-        }
-        float mn = m;
-#pragma unroll
-        for (int u = 0; u < DEC_UNROLL; ++u) mn = fmaxf(mn, s[u]);
-        const float mref = (mn == -INFINITY) ? 0.f : mn;   // half-warp without a valid key yet: everything stays 0
-        const float corr = exp2f(m - mref);               // m = -inf -> 0
-        m = mn;
-        lsum *= corr;
-#pragma unroll
-        for (int t = 0; t < 8; ++t) acc[t] *= corr;
-#pragma unroll
-        for (int u = 0; u < DEC_UNROLL; ++u) {
-            const float p = exp2f(s[u] - mref);
-            lsum += p;
-            const float pr = bf16_round(p);   // same rounding point as the tensor-core kernel's P operand
-            const __nv_bfloat162* v2 = reinterpret_cast<const __nv_bfloat162*>(&vv[u]);
-#pragma unroll
-            for (int t = 0; t < 4; ++t) {
-                const float2 f = __bfloat1622float2(v2[t]);
-                acc[2 * t] += pr * f.x;
-                acc[2 * t + 1] += pr * f.y;
-            }
-        }
-#pragma unroll
-        for (int u = 0; u < DEC_UNROLL; ++u) kcur[u] = knext[u];
-    }
-    __shared__ float sm_m[DEC_WARPS * 2], sm_l[DEC_WARPS * 2], sm_acc[DEC_WARPS * 2][D];
-    __shared__ float peer_m[DEC_SPLIT], peer_l[DEC_SPLIT], peer_acc[DEC_SPLIT][D];   // written by every rank into rank 0
-    const int slot = warp * 2 + grp;
-    if (l == 0) { sm_m[slot] = m; sm_l[slot] = lsum; }
-#pragma unroll
-    for (int t = 0; t < 8; ++t) sm_acc[slot][l * 8 + t] = acc[t];
-    __syncthreads();
-    cluster_wait();   // pairs with the arrive at kernel entry: every CTA of the cluster has started
-    // CTA-level merge -> (M, den, num[D]) sent to the leader CTA's shared memory (distributed shared memory)
-    float* r_m = cluster.map_shared_rank(peer_m, 0);
-    float* r_l = cluster.map_shared_rank(peer_l, 0);
-    float* r_acc = cluster.map_shared_rank(&peer_acc[0][0], 0);
-    for (int d = threadIdx.x; d < D; d += blockDim.x) {
-        float M = -INFINITY;
-#pragma unroll
-        for (int w = 0; w < DEC_WARPS * 2; ++w) M = fmaxf(M, sm_m[w]);
-        float num = 0.f, den = 0.f;
-#pragma unroll
-        for (int w = 0; w < DEC_WARPS * 2; ++w) {
-            const float c = (sm_m[w] == -INFINITY) ? 0.f : exp2f(sm_m[w] - M);
-            num += c * sm_acc[w][d];
-            den += c * sm_l[w];
-        }
-        r_acc[crank * D + d] = num;
-        if (d == 0) { r_m[crank] = M; r_l[crank] = den; }
-    }
-    cluster.sync();
-    if (crank == 0) {
-        for (int d = threadIdx.x; d < D; d += blockDim.x) {
-            float M = -INFINITY;
-#pragma unroll
-            for (int r = 0; r < DEC_SPLIT; ++r) M = fmaxf(M, peer_m[r]);
-            float num = 0.f, den = 0.f;
-#pragma unroll
-            for (int r = 0; r < DEC_SPLIT; ++r) {
-                const float c = (peer_m[r] == -INFINITY) ? 0.f : exp2f(peer_m[r] - M);
-                num += c * peer_acc[r][d];
-                den += c * peer_l[r];
-            }
-            out[((long long)b * H + h) * D + d] = __float2bfloat16_rn(den > 0.f ? num / den : 0.f);
-        }
-    }
-}
-
-
-// ------------------------------------------------------------------------------------------------------------------
-// Same decode attention with the K/V stream staged by the TMA engine: per CTA one producer lane issues 1-D bulk copies of
-// DT_KEYS consecutive K rows and V rows (contiguous in the [B,H,cap,D] cache) into a DT_STAGES-deep shared-memory ring,
-// the DEC_WARPS consumer warps run the identical per-key arithmetic out of shared memory (same key->half-warp assignment
-// and the same groups of 4 keys per online-softmax update as decode_attention_kernel<128,4>, so results are bit-identical).
-// Bytes in flight no longer depend on registers/occupancy: 8 resident CTAs x 24 KB per SM.
 constexpr int DT_UNROLL = 4;
 constexpr int DT_KEYS = DEC_WARPS * 2 * DT_UNROLL;   // keys per stage (16)
 #ifndef GROMA_DT_STAGES
@@ -451,7 +296,9 @@ __global__ void __cluster_dims__(DEC_SPLIT, 1, 1) __launch_bounds__((DEC_WARPS +
     __shared__ float sm_m[DEC_WARPS * 2], sm_l[DEC_WARPS * 2], sm_acc[DEC_WARPS * 2][D];
     __shared__ float peer_m[DEC_SPLIT], peer_l[DEC_SPLIT], peer_acc[DEC_SPLIT][D];
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    cluster_arrive_relaxed();   // see decode_attention_kernel: waited on right before the first remote shared-memory store
+    // distributed-shared-memory rule: a CTA may only touch a peer's shared memory once that peer is known to be running.
+    // Arrive now, wait just before the first remote store -- the barrier latency hides behind the key loop.
+    cluster_arrive_relaxed();
     if (threadIdx.x == 0) {
         for (int s = 0; s < DT_STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], DEC_WARPS); }
         fence_barrier_init();
@@ -650,32 +497,17 @@ GROMA_API int32_t groma_decode_attention(const void* q, const void* cache_k, con
     if (!q || !cache_k || !cache_v || !out || !kv_len || B <= 0 || H <= 0) return GROMA_ERR_ARG;
     if (D != 128) return GROMA_ERR_UNSUPPORTED;
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(H * gb::DEC_SPLIT, B); cfg.blockDim = dim3(gb::DEC_WARPS * 32); cfg.dynamicSmemBytes = 0;
+    cfg.gridDim = dim3(H * gb::DEC_SPLIT, B); cfg.blockDim = dim3((gb::DEC_WARPS + 1) * 32); cfg.dynamicSmemBytes = 0;
     cfg.stream = reinterpret_cast<cudaStream_t>(stream);
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     if (pdl) { cfg.attrs = attr; cfg.numAttrs = 1; }
-    static int unroll = 0;   // loads in flight per lane = 2 * unroll x 16 B; GROMA_DEC_UNROLL overrides for tuning
-    if (!unroll) { const char* ev = getenv("GROMA_DEC_UNROLL"); unroll = ev ? atoi(ev) : 4; }
-    auto Q = reinterpret_cast<const __nv_bfloat16*>(q);
-    auto K = reinterpret_cast<const __nv_bfloat16*>(cache_k);
-    auto V = reinterpret_cast<const __nv_bfloat16*>(cache_v);
-    auto O = reinterpret_cast<__nv_bfloat16*>(out);
-    const float sl2 = scale * 1.4426950408889634f;
-    cudaError_t e;
-    static int use_tma = -1;   // default: K/V staged through the TMA ring (decode_attention_tma_kernel); GROMA_DEC_ATTN_TMA=0 = LDG kernel
-    if (use_tma < 0) { const char* ev = getenv("GROMA_DEC_ATTN_TMA"); use_tma = ev ? atoi(ev) : 1; }
-    if (use_tma) {
-        cfg.blockDim = dim3((gb::DEC_WARPS + 1) * 32);
-        e = cudaLaunchKernelEx(&cfg, gb::decode_attention_tma_kernel<128, false>, Q, const_cast<__nv_bfloat16*>(K),
-                               const_cast<__nv_bfloat16*>(V), O, kv_len, (int)H, (long long)cap, sl2, gb::DecodeRopeArgs{});
-        return e == cudaSuccess ? GROMA_OK : GROMA_ERR_CUDA;
-    }
-    if (unroll == 8) e = cudaLaunchKernelEx(&cfg, gb::decode_attention_kernel<128, 8>, Q, K, V, O, kv_len, (int)H, (long long)cap, sl2);
-    else if (unroll == 6) e = cudaLaunchKernelEx(&cfg, gb::decode_attention_kernel<128, 6>, Q, K, V, O, kv_len, (int)H, (long long)cap, sl2);
-    else if (unroll == 2) e = cudaLaunchKernelEx(&cfg, gb::decode_attention_kernel<128, 2>, Q, K, V, O, kv_len, (int)H, (long long)cap, sl2);
-    else e = cudaLaunchKernelEx(&cfg, gb::decode_attention_kernel<128, 4>, Q, K, V, O, kv_len, (int)H, (long long)cap, sl2);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, gb::decode_attention_tma_kernel<128, false>, reinterpret_cast<const __nv_bfloat16*>(q),
+                                       reinterpret_cast<__nv_bfloat16*>(const_cast<void*>(cache_k)),
+                                       reinterpret_cast<__nv_bfloat16*>(const_cast<void*>(cache_v)),
+                                       reinterpret_cast<__nv_bfloat16*>(out), kv_len, (int)H, (long long)cap,
+                                       scale * 1.4426950408889634f, gb::DecodeRopeArgs{});
     return e == cudaSuccess ? GROMA_OK : GROMA_ERR_CUDA;
 }
 

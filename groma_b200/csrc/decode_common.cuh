@@ -36,14 +36,6 @@ __device__ __forceinline__ void splitk_pairs(const float* __restrict__ ws, int S
     }
 }
 
-__device__ __forceinline__ void splitk_pair(const float* __restrict__ ws, int S, int B, int N, int b, int col, int j, int half,
-                                            float& a1, float& a2) {
-    const int c[1] = {col};
-    float x1[1], x2[1];
-    splitk_pairs<1>(ws, S, B, N, b, c, j, half, x1, x2);
-    a1 = x1[0]; a2 = x2[0];
-}
-
 // sum over s < S of the float4 at p + s * stride (stride in floats), up to U loads in flight per pass
 template <int U = 16>
 __device__ __forceinline__ float4 splitk_sum4(const float* __restrict__ p, long long stride, int S) {

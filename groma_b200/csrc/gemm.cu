@@ -1,6 +1,5 @@
 // Host launcher for the tcgen05 GEMM / implicit-GEMM conv and the split-K reduce epilogue.
 // C ABI: see include/groma_b200.h (groma_gemm_bf16, groma_splitk_reduce).
-#include <cstdlib>
 #include "gemm_tcgen05.cuh"
 #include "capi_common.h"
 
@@ -83,9 +82,9 @@ static int launch_gemm(const GemmParams& p, cudaStream_t stream) {
     const int n_tiles = (p.N + BN - 1) / BN;
     const int work = m_tiles * n_tiles * p.split_k;
     // BN = 16 (decode swap-AB): 4-stage ring, two CTAs per SM -- one CTA's tile epilogue / tile switch overlaps the other's
-    // streaming (measured: GEMM-only decode graph 2.34 -> 2.25 ms vs one 8-stage CTA per SM).  GROMA_GEMM_CTAS_PER_SM overrides.
-    static const int per_sm16 = [] { const char* e = getenv("GROMA_GEMM_CTAS_PER_SM"); return e ? atoi(e) : 2; }();
-    const int slots = num_sms() * ((BN == 16 && per_sm16 > 0) ? per_sm16 : 1);
+    // streaming (measured: GEMM-only decode graph 2.34 -> 2.25 ms vs one 8-stage CTA per SM).  GromaEngine._decode_splits
+    // sizes the decode split-K factors for these 2 CTAs per SM: change both together.
+    const int slots = num_sms() * (BN == 16 ? 2 : 1);
     const int grid = work < slots ? work : slots;
     if (p.flags & GF_PDL) {
         cudaLaunchConfig_t cfg = {};
@@ -170,7 +169,7 @@ static int32_t gemm_impl(const void* A, int64_t a_rows, int64_t lda, const void*
                          int64_t ldb, int32_t M, int32_t N, int32_t K, int32_t num_taps,
                          const int32_t* a_row_off, void* out, int64_t ld_m, int64_t ld_n, int32_t flags,
                          int32_t act, const float* bias, const float* gamma, const void* residual,
-                         float* ws, int32_t split_k, int32_t* tile_counters, int32_t conv_hp, int32_t conv_wp,
+                         float* ws, int32_t split_k, int32_t conv_hp, int32_t conv_wp,
                          int32_t block_n, void* stream, const RopeEpilogue* rope) {
     if (!A || !B || M <= 0 || N <= 0 || K <= 0) return GROMA_ERR_ARG;
     if (((flags & GF_ROPE_QKV) != 0) != (rope != nullptr)) return GROMA_ERR_ARG;
@@ -181,11 +180,9 @@ static int32_t gemm_impl(const void* A, int64_t a_rows, int64_t lda, const void*
     if (split_k > 1 && !(flags & GF_PARTIAL)) return GROMA_ERR_ARG;
     if ((flags & GF_PARTIAL) && !ws) return GROMA_ERR_ARG;
     if (!(flags & GF_PARTIAL) && !out) return GROMA_ERR_ARG;
-    if (tile_counters && (!(flags & GF_PARTIAL) || !out)) return GROMA_ERR_ARG;
     if (act == ACT_SWIGLU && !(flags & GF_BIAS_ALONG_M) && (N & 1)) return GROMA_ERR_ARG;
     if (act == ACT_SWIGLU && (flags & GF_BIAS_ALONG_M) && (M & 1)) return GROMA_ERR_ARG;
     if (num_taps > 1 && (K % GEMM_BK) != 0) return GROMA_ERR_ARG;
-    if ((flags & GF_A_TILED) && (num_taps != 1 || lda != GEMM_BK)) return GROMA_ERR_ARG;
 
     int bn = block_n;
     if (bn == 0) {
@@ -200,9 +197,8 @@ static int32_t gemm_impl(const void* A, int64_t a_rows, int64_t lda, const void*
             if (bn == 128 && m_tiles * ((N + 127) / 128) * split_k < num_sms() / 2 && N >= 128) bn = 64;
         }
     }
-    if (tile_counters && gemm_epi_warps(bn == 512 ? 256 : bn) != 4) return GROMA_ERR_UNSUPPORTED;   // fused split-K finish: narrow (decode) tiles only
     GemmParams p;
-    int rc = make_tma_2d(&p.tma_a, A, (uint64_t)a_rows, (flags & GF_A_TILED) ? (uint64_t)GEMM_BK : (uint64_t)K, (uint64_t)lda, GEMM_BM);
+    int rc = make_tma_2d(&p.tma_a, A, (uint64_t)a_rows, (uint64_t)K, (uint64_t)lda, GEMM_BM);
     if (rc) return rc;
     rc = make_tma_2d(&p.tma_b, B, (uint64_t)b_rows, (uint64_t)K * num_taps, (uint64_t)ldb, bn == 512 ? 128u : (uint32_t)bn);
     if (rc) return rc;
@@ -211,7 +207,7 @@ static int32_t gemm_impl(const void* A, int64_t a_rows, int64_t lda, const void*
     p.split_k = split_k; p.flags = flags; p.act = act;
     p.out = out; p.ld_m = ld_m; p.ld_n = ld_n;
     p.bias = bias; p.gamma = gamma; p.residual = reinterpret_cast<const __nv_bfloat16*>(residual);
-    p.ws = ws; p.conv_hp = conv_hp; p.conv_wp = conv_wp; p.tile_counters = tile_counters;
+    p.ws = ws; p.conv_hp = conv_hp; p.conv_wp = conv_wp;
     p.rope_cos = p.rope_sin = nullptr; p.rope_k = p.rope_v = nullptr; p.rope_T = 1; p.rope_H = 1; p.rope_pos0 = 0; p.rope_cap = 0;
     if (rope) {
         if (bn != 256 && bn != 512) return GROMA_ERR_UNSUPPORTED;   // one head (128 columns) per epilogue warp needs the 256-wide tile
@@ -219,14 +215,9 @@ static int32_t gemm_impl(const void* A, int64_t a_rows, int64_t lda, const void*
         p.rope_k = reinterpret_cast<__nv_bfloat16*>(rope->cache_k); p.rope_v = reinterpret_cast<__nv_bfloat16*>(rope->cache_v);
         p.rope_T = rope->T; p.rope_H = rope->H; p.rope_pos0 = rope->pos0; p.rope_cap = rope->cap;
     }
-    {
-        // early release of the dependent grid (measured: decode step 4.49 -> 4.40 ms); GROMA_GEMM_EARLY_TRIGGER=0 disables
-        static const int early = [] { const char* e = getenv("GROMA_GEMM_EARLY_TRIGGER"); return e ? atoi(e) : 1; }();
-        p.early_trigger = (flags & GF_PDL) ? early : 0;
-    }
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     if (bn == 512) {   // block_n = 512 selects the 2-CTA (256 x 256 per cluster) kernel
-        if (split_k != 1 || (flags & (GF_PARTIAL | GF_PDL | GF_A_TILED))) return GROMA_ERR_ARG;
+        if (split_k != 1 || (flags & (GF_PARTIAL | GF_PDL))) return GROMA_ERR_ARG;
         return launch_gemm_2cta(p, st);
     }
     switch (bn) {
@@ -243,11 +234,11 @@ GROMA_API int32_t groma_gemm_bf16(const void* A, int64_t a_rows, int64_t lda, co
                                    int64_t ldb, int32_t M, int32_t N, int32_t K, int32_t num_taps,
                                    const int32_t* a_row_off, void* out, int64_t ld_m, int64_t ld_n, int32_t flags,
                                    int32_t act, const float* bias, const float* gamma, const void* residual,
-                                   float* ws, int32_t split_k, int32_t* tile_counters, int32_t conv_hp, int32_t conv_wp,
+                                   float* ws, int32_t split_k, int32_t conv_hp, int32_t conv_wp,
                                    int32_t block_n, void* stream) {
     if (flags & GF_ROPE_QKV) return GROMA_ERR_ARG;   // that epilogue has its own entry point below
     return gemm_impl(A, a_rows, lda, B, b_rows, ldb, M, N, K, num_taps, a_row_off, out, ld_m, ld_n, flags, act, bias, gamma,
-                     residual, ws, split_k, tile_counters, conv_hp, conv_wp, block_n, stream, nullptr);
+                     residual, ws, split_k, conv_hp, conv_wp, block_n, stream, nullptr);
 }
 
 // LLaMA attention input in one launch: x [B*T, K] @ Wqkv^T [3*H*128, K] with rotate-half RoPE on q/k and the KV-cache
@@ -268,7 +259,7 @@ GROMA_API int32_t groma_gemm_qkv_rope(const void* x, int64_t ldx, const void* w_
     const long long M = (long long)B * T;
     if (M > 0x7fffffffLL) return GROMA_ERR_ARG;
     return gemm_impl(x, M, ldx, w_qkv, 3LL * H * D, ldw, (int32_t)M, 3 * H * D, K, 1, nullptr, q_out, (int64_t)H * D, 1,
-                     GF_ROPE_QKV, ACT_NONE, nullptr, nullptr, nullptr, nullptr, 1, nullptr, 0, 0, block_n, stream, &r);
+                     GF_ROPE_QKV, ACT_NONE, nullptr, nullptr, nullptr, nullptr, 1, 0, 0, block_n, stream, &r);
 }
 
 GROMA_API int32_t groma_splitk_reduce(const float* ws, int32_t splits, int32_t M, int32_t N, int32_t act,

@@ -28,8 +28,8 @@ enum GemmFlags : int {
     GF_PARTIAL = 4,       // store raw fp32 accumulators to ws[split][m][n] (split-K / deferred epilogue)
     GF_CONV_ROWS = 8,     // rows are pixels of zero-bordered [img][hp][wp] maps: skip border rows
     GF_CONV_COMPACT = 16, // with GF_CONV_ROWS: write row index of the un-padded [img][h][w] layout
-    GF_A_TILED = 32,      // A is pre-tiled in HBM: [m_tile][k_block][128 rows][64 cols] -> every TMA load is one contiguous 16 KB
-    GF_PDL = 64,          // launched with programmatic stream serialisation: A (weights) is prefetched before griddepcontrol.wait
+    GF_PDL = 64,          // launched with programmatic stream serialisation: A (weights) is prefetched before griddepcontrol.wait,
+                          // and the dependent grid is released at kernel start (it parks at its own griddepcontrol.wait)
     GF_PARTIAL_T = 128,   // with GF_PARTIAL: partials stored transposed, ws[split][n][m] (swap-AB decode: token-major rows)
     GF_ROPE_QKV = 256,    // fused LLaMA qkv projection: rotate q/k (RoPE) in the epilogue, q -> out, k/v -> the KV cache (256-wide tiles, D = 128)
 };
@@ -50,8 +50,6 @@ struct GemmParams {
     const __nv_bfloat16* residual;  // same strides as out, or null
     float* ws;             // fp32 partials [split][M][N] when GF_PARTIAL
     int conv_hp, conv_wp;  // padded map dims for GF_CONV_ROWS
-    int* tile_counters;    // GF_PARTIAL + non-null: the CTA that completes a tile's last split reduces ws and runs the epilogue
-    int early_trigger;     // GF_PDL: release the dependent grid at kernel start (it parks at its own griddepcontrol.wait)
     // GF_ROPE_QKV: rows = (sequence b, token t) with t < rope_T; columns = [q | k | v] x [rope_H heads] x [128]
     const float* rope_cos;  // fp32 [max_pos, 64]
     const float* rope_sin;
@@ -60,10 +58,6 @@ struct GemmParams {
     int rope_T, rope_H, rope_pos0;
     long long rope_cap;
 };
-
-#ifndef GROMA_EPI_V2
-#define GROMA_EPI_V2 1   // pipelined epilogue (A/B: tools/build_variants.sh epi1 -DGROMA_EPI_V2=0)
-#endif
 
 template <int BN, int CG = 1>
 struct GemmCfg {
@@ -120,11 +114,9 @@ __global__ void __launch_bounds__(gemm_threads(BN), 1) gemm_bf16_tcgen05_kernel(
     uint32_t* tmem_holder = reinterpret_cast<uint32_t*>(tempty_bar + 2);
     constexpr int STG_WARP_BYTES = 32 * 80 + 32 * 8;  // 32 rows x (64 B + 16 B pad) + 32 output-row indices
     uint8_t* stage_base = reinterpret_cast<uint8_t*>(tmem_holder + 4);
-    volatile int* finish_flag = reinterpret_cast<volatile int*>(tmem_holder + 1);
 
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
-    constexpr bool EPI2 = GROMA_EPI_V2 != 0;
 
     const int crank = (CG == 2) ? (int)cluster_ctarank() : 0;     // rank inside the CTA pair
     const int wid0 = blockIdx.x / CG, wstride = gridDim.x / CG;     // work is distributed over clusters
@@ -161,14 +153,13 @@ __global__ void __launch_bounds__(gemm_threads(BN), 1) gemm_bf16_tcgen05_kernel(
     const uint32_t tmem_base = *tmem_holder;
     // Dependents only touch this grid's results after their own griddepcontrol.wait (= this grid complete and flushed), so
     // releasing them now is safe; it lets the next kernels become resident and the next GEMM stream its weights early.
-    if (p.early_trigger) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    if (p.flags & GF_PDL) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
 
     if (warp == 0) {
         // ===================== TMA producer =====================
         if (lane == 0) {
             int stage = 0;
             uint32_t phase = 0;
-            const bool a_tiled = (p.flags & GF_A_TILED) != 0;
             // work iterator over this CTA's (work item, k-iteration) pairs
             int w = wid0, it = 0, it1 = 0, m_blk = 0, n_blk = 0;
             auto load_work = [&]() {
@@ -184,10 +175,6 @@ __global__ void __launch_bounds__(gemm_threads(BN), 1) gemm_bf16_tcgen05_kernel(
                 }
                 return false;
             };
-            auto a_coords = [&](int tap, int kb, int& c0, int& c1) {
-                if (a_tiled) { c0 = 0; c1 = (m_blk * kb_per_tap + kb) * GEMM_BM; }
-                else { c0 = kb * GEMM_BK; c1 = m_blk * GEMM_BM + p.a_row_off[tap]; }
-            };
             bool have = load_work();
             if ((CG == 1) && (p.flags & GF_PDL)) {
                 // The A operand (weights) does not depend on the previous kernel: fill the ring with A tiles first, only then
@@ -196,10 +183,8 @@ __global__ void __launch_bounds__(gemm_threads(BN), 1) gemm_bf16_tcgen05_kernel(
                 int issued = 0;
                 while (have && issued < STAGES) {
                     const int tap = it / kb_per_tap, kb = it - tap * kb_per_tap;
-                    int c0, c1;
-                    a_coords(tap, kb, c0, c1);
                     mbar_expect_tx(&full_bar[issued], Cfg::STAGE_BYTES);
-                    tma_load_2d(smem + issued * Cfg::STAGE_BYTES, &p.tma_a, &full_bar[issued], c0, c1);
+                    tma_load_2d(smem + issued * Cfg::STAGE_BYTES, &p.tma_a, &full_bar[issued], kb * GEMM_BK, m_blk * GEMM_BM + p.a_row_off[tap]);
                     bc0[issued] = tap * p.K + kb * GEMM_BK;
                     bc1[issued] = n_blk * BN;
                     ++issued;
@@ -215,8 +200,7 @@ __global__ void __launch_bounds__(gemm_threads(BN), 1) gemm_bf16_tcgen05_kernel(
                 mbar_wait(&empty_bar[stage], phase ^ 1);
                 uint8_t* sa = smem + stage * Cfg::STAGE_BYTES;
                 uint8_t* sb = sa + Cfg::A_BYTES;
-                int c0, c1;
-                a_coords(tap, kb, c0, c1);
+                const int c0 = kb * GEMM_BK, c1 = m_blk * GEMM_BM + p.a_row_off[tap];
                 if constexpr (CG == 2) {
                     // both CTAs credit the LEADER's full barrier: the leader arms it with the bytes of the whole pair
                     if (crank == 0) mbar_expect_tx(&full_bar[stage], 2 * Cfg::STAGE_BYTES);
@@ -285,10 +269,6 @@ __global__ void __launch_bounds__(gemm_threads(BN), 1) gemm_bf16_tcgen05_kernel(
             m_blk = m_blk * CG + crank;
             const int it0 = split * iters_per_split;
             const bool has_work = it0 < total_iters;  // an empty split contributes zeros
-            if constexpr (!EPI2) {
-                mbar_wait(&tfull_bar[acc], acc_phase);
-                tc_fence_after();
-            }
             const int row = m_blk * GEMM_BM + q * 32 + lane;
             bool row_ok = row < p.M;
             long long out_row = row;
@@ -311,12 +291,12 @@ __global__ void __launch_bounds__(gemm_threads(BN), 1) gemm_bf16_tcgen05_kernel(
             const uint32_t stg_s = smem_u32(stg);
             bool released = false;
             int c_first = col_lo;
-            // EPI2: the bias / LayerScale values of this warp's columns are fetched ONCE per tile (one float4 of each per lane, while
+            // The bias / LayerScale values of this warp's columns are fetched ONCE per tile (one float4 of each per lane, while
             // the tile's MMAs are still running) into a per-warp kilobyte of shared memory and read back as broadcast LDS.  As
             // per-chunk global loads (8 + 8 LDG.128 per 32 columns) they missed the ~28 KB of L1 left beside 220 KB of shared memory
             // -- the residual / output stream evicts them -- and every chunk paid a chain of L2 round trips.
             const uint32_t bg_s = smem_u32(stage_base + Cfg::EPW * STG_WARP_BYTES + (warp - 2) * 1024);
-            const bool use_bg = EPI2 && !bias_m && !partial && (p.bias != nullptr || p.gamma != nullptr);
+            const bool use_bg = !bias_m && !partial && (p.bias != nullptr || p.gamma != nullptr);
             if (use_bg) {
                 __syncwarp();   // the previous tile's readers are done with the buffer
                 const int c = lane * 4;
@@ -333,19 +313,17 @@ __global__ void __launch_bounds__(gemm_threads(BN), 1) gemm_bf16_tcgen05_kernel(
                 }
                 __syncwarp();
             }
-            if constexpr (EPI2) {
-                // While the tile's MMAs are still running: pull this lane's residual row segment (BN / EPH columns) towards L2, so
-                // the epilogue's residual loads are L2 hits instead of exposed DRAM round trips (the short-K ViT projections spent
-                // their epilogue in stall_long_sb on exactly these loads)
-                if (p.residual != nullptr && !partial && p.ld_n == 1 && row_ok) {
-                    const char* rp = reinterpret_cast<const char*>(p.residual + out_row * p.ld_m + (long long)n_blk * BN + col_lo);
+            // While the tile's MMAs are still running: pull this lane's residual row segment (BN / EPH columns) towards L2, so
+            // the epilogue's residual loads are L2 hits instead of exposed DRAM round trips (the short-K ViT projections spent
+            // their epilogue in stall_long_sb on exactly these loads)
+            if (p.residual != nullptr && !partial && p.ld_n == 1 && row_ok) {
+                const char* rp = reinterpret_cast<const char*>(p.residual + out_row * p.ld_m + (long long)n_blk * BN + col_lo);
 #pragma unroll
-                    for (int b = 0; b < (BN / EPH) * 2; b += 128)
-                        if (n_blk * BN + col_lo + (b >> 1) < p.N) asm volatile("prefetch.global.L2 [%0];" ::"l"(rp + b));
-                }
-                mbar_wait(&tfull_bar[acc], acc_phase);
-                tc_fence_after();
+                for (int b = 0; b < (BN / EPH) * 2; b += 128)
+                    if (n_blk * BN + col_lo + (b >> 1) < p.N) asm volatile("prefetch.global.L2 [%0];" ::"l"(rp + b));
             }
+            mbar_wait(&tfull_bar[acc], acc_phase);
+            tc_fence_after();
             if constexpr (BN == 256 && Cfg::EPW == 8) {
                 if (p.flags & GF_ROPE_QKV) {
                     // This warp's 128 columns are exactly one head of q, k or v.  The projection is rounded to bf16 first (what the
@@ -407,13 +385,13 @@ __global__ void __launch_bounds__(gemm_threads(BN), 1) gemm_bf16_tcgen05_kernel(
                     }
                 }
             }
-            // EPI2: the residual row segment of a chunk is requested BEFORE its accumulators are read (the two latencies overlap),
+            // The residual row segment of a chunk is requested BEFORE its accumulators are read (the two latencies overlap),
             // and the accumulator stage goes back to the MMA warp as soon as the last chunk sits in registers, not after it has
             // been stored.  (Double-buffering the tcgen05.ld across chunks was tried as well: the 32 extra registers pushed
             // loop invariants into local memory, and with ~28 KB of L1 those reloads are L2 round trips -- ncu showed every
             // long-scoreboard stall of the epilogue on them; profiles/r02_gemm_epilogue_v2.md.)
             const uint32_t tbase = tmem_base + (uint32_t(q * 32) << 16) + uint32_t(acc * BN);
-            const bool res_vec_ok = EPI2 && p.residual != nullptr && !partial && p.ld_n == 1 && (p.ld_m & 7) == 0;
+            const bool res_vec_ok = p.residual != nullptr && !partial && p.ld_n == 1 && (p.ld_m & 7) == 0;
 #pragma unroll 1
             for (int c0 = c_first; c0 < col_hi; c0 += CHUNK) {
                 uint32_t v[32];
@@ -429,14 +407,12 @@ __global__ void __launch_bounds__(gemm_threads(BN), 1) gemm_bf16_tcgen05_kernel(
                 __syncwarp();  // tcgen05.ld is .sync.aligned (and orders the staging buffer reuse)
                 if (CHUNK == 32) tmem_ld32(tbase + c0, v); else tmem_ld16(tbase + c0, v);
                 tmem_ld_wait();
-                if constexpr (EPI2) {
-                    if (c0 + CHUNK >= col_hi && !(partial && p.tile_counters != nullptr)) {
-                        // every column of this warp's share is in registers: release the accumulator stage now
-                        tc_fence_before();
-                        __syncwarp();
-                        if (lane == 0) { if constexpr (CG == 2) mbar_arrive_cta(&tempty_bar[acc], 0); else mbar_arrive(&tempty_bar[acc]); }
-                        released = true;
-                    }
+                if (c0 + CHUNK >= col_hi) {
+                    // every column of this warp's share is in registers: release the accumulator stage now
+                    tc_fence_before();
+                    __syncwarp();
+                    if (lane == 0) { if constexpr (CG == 2) mbar_arrive_cta(&tempty_bar[acc], 0); else mbar_arrive(&tempty_bar[acc]); }
+                    released = true;
                 }
                 if (!staged && !active) continue;
                 if (!has_work) {
@@ -550,7 +526,7 @@ __global__ void __launch_bounds__(gemm_threads(BN), 1) gemm_bf16_tcgen05_kernel(
                         }
                     }
                 }
-                if (EPI2 && staged && CHUNK == 32 && !swiglu && n0 + CHUNK <= p.N) {
+                if (staged && CHUNK == 32 && !swiglu && n0 + CHUNK <= p.N) {
                     // 32 rows x 64 B through shared memory: 4 x STS.128 (own row), 4 x LDS.128 (4 lanes per row, 8 rows per
                     // instruction), 4 x STG.128 writing 8 complete 64-byte row segments each -- no generic-address accesses and
                     // no load -> branch -> load -> store chain per slot
@@ -621,75 +597,6 @@ __global__ void __launch_bounds__(gemm_threads(BN), 1) gemm_bf16_tcgen05_kernel(
                     __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(p.out) + obase;
                     _Pragma("unroll") for (int j = 0; j < CHUNK; ++j) if (j < out_cols && no0 + j < NO) dst[(long long)j * p.ld_n] = __float2bfloat16_rn(f[j]);
                 }
-            }
-            // ---- fused split-K finish: the last CTA to deliver a partial of this tile sums all splits (fixed order, so the
-            //      result is deterministic) and runs the epilogue -- no separate reduce launch on the decode path
-            if (partial && p.tile_counters != nullptr) {
-                // (host side refuses tile_counters for tiles >= 128 columns: this finish assumes the 128-thread epilogue of narrow tiles)
-                tc_fence_before();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&tempty_bar[acc]);   // TMEM no longer needed: let the MMA warp run ahead
-                __threadfence();
-                asm volatile("bar.sync 1, 128;" ::: "memory");
-                if (warp == 2 && lane == 0) {
-                    const int old = atomicAdd(p.tile_counters + tile, 1);
-                    const int last = (old == p.split_k - 1) ? 1 : 0;
-                    if (last) p.tile_counters[tile] = 0;        // re-arm for the next launch / graph replay
-                    *finish_flag = last;
-                }
-                asm volatile("bar.sync 1, 128;" ::: "memory");
-                if (*finish_flag) {
-                    __threadfence();
-                    const bool swiglu_m = (p.act == ACT_SWIGLU);   // pairs along M: rows (2j, 2j+1) = (gate_j, up_j)
-                    const float bm = (row_ok && p.bias && bias_m) ? p.bias[row] : 0.0f;
-                    const float gm = (row_ok && p.gamma && bias_m) ? p.gamma[row] : 1.0f;
-#pragma unroll 1
-                    for (int c0 = 0; c0 < BN; c0 += 16) {
-                        const int n0 = n_blk * BN + c0;
-                        if (n0 >= p.N) break;
-                        float a16[16];
-#pragma unroll
-                        for (int j = 0; j < 16; ++j) a16[j] = 0.0f;
-                        if (row_ok) {
-                            for (int sp = 0; sp < p.split_k; ++sp) {
-                                const float* src = p.ws + ((long long)sp * p.M + out_row) * p.N + n0;
-                                if ((p.N & 3) == 0 && n0 + 16 <= p.N) {
-#pragma unroll
-                                    for (int j = 0; j < 16; j += 4) {
-                                        const float4 t4 = __ldcg(reinterpret_cast<const float4*>(src + j));
-                                        a16[j] += t4.x; a16[j + 1] += t4.y; a16[j + 2] += t4.z; a16[j + 3] += t4.w;
-                                    }
-                                } else {
-#pragma unroll
-                                    for (int j = 0; j < 16; ++j) if (n0 + j < p.N) a16[j] += __ldcg(src + j);
-                                }
-                            }
-                        }
-#pragma unroll
-                        for (int j = 0; j < 16; ++j) {
-                            const int n = n0 + j;
-                            float x = a16[j];
-                            if (p.bias) x += bias_m ? bm : (n < p.N ? p.bias[n] : 0.0f);
-                            if (swiglu_m) {
-                                const float other = __shfl_xor_sync(0xffffffffu, x, 1);
-                                if (row_ok && !(row & 1) && n < p.N)
-                                    reinterpret_cast<__nv_bfloat16*>(p.out)[(out_row >> 1) * p.ld_m + (long long)n * p.ld_n] =
-                                        __float2bfloat16_rn(silu(x) * other);
-                                continue;
-                            }
-                            x = apply_act(x, p.act);
-                            if (p.gamma) x *= bias_m ? gm : (n < p.N ? p.gamma[n] : 1.0f);
-                            if (row_ok && n < p.N) {
-                                const long long o = out_row * p.ld_m + (long long)n * p.ld_n;
-                                if (p.residual) x += __bfloat162float(p.residual[o]);
-                                if (out_f32) reinterpret_cast<float*>(p.out)[o] = x;
-                                else reinterpret_cast<__nv_bfloat16*>(p.out)[o] = __float2bfloat16_rn(x);
-                            }
-                        }
-                    }
-                }
-                if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-                continue;
             }
             // release this accumulator stage back to the MMA warp (of the leader CTA)
             if (!released) {

@@ -11,17 +11,6 @@ namespace gb {
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));
 }
-__device__ __forceinline__ uint32_t lane_id() { return threadIdx.x & 31; }
-
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred = 0;
-    asm volatile(
-        "{\n\t.reg .pred P;\n\t"
-        "elect.sync _|P, 0xffffffff;\n\t"
-        "selp.u32 %0, 1, 0, P;\n\t}\n"
-        : "=r"(pred));
-    return pred != 0;
-}
 
 // ---------------------------------------------------------------- mbarrier
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
@@ -29,9 +18,6 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
 }
 __device__ __forceinline__ void fence_barrier_init() {
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void fence_proxy_async() {
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 }
 __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes)
@@ -137,9 +123,6 @@ __device__ __forceinline__ uint4 ld_shared_v4(uint32_t addr) {
     uint4 v;
     asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr) : "memory");
     return v;
-}
-__device__ __forceinline__ void st_shared_b64(uint32_t addr, long long v) {
-    asm volatile("st.shared.b64 [%0], %1;" ::"r"(addr), "l"(v) : "memory");
 }
 __device__ __forceinline__ long long ld_shared_b64(uint32_t addr) {
     long long v;

@@ -9,7 +9,6 @@ replaces are cited at the methods (paths relative to the FoundationVision/Groma 
 from __future__ import annotations
 
 import math
-import os
 from typing import Dict, List, Optional, Sequence
 
 import torch
@@ -24,6 +23,8 @@ def _cat(*ts):
 
 
 class GromaEngine:
+    use_megakernel = False   # read by bench.py's decode roofline; there is no persistent decode kernel
+
     def __init__(self, cfg: PathConfig, state_dict: Dict[str, torch.Tensor], device: str = "cuda", detector_only: bool = False):
         """state_dict: any mapping key -> tensor with the reference's parameter names (a lazy `ShardedStateDict` reads each
         tensor from its shard exactly when it is packed).  detector_only: a `CustomDDETRModel` checkpoint (keys without the
@@ -40,25 +41,12 @@ class GromaEngine:
         self.kv = None
         self.stages: Dict[str, torch.Tensor] = {}
         self.keep_stages = False
-        self.fused_splitk = False
-        self.decode_tiled = os.environ.get("GROMA_DECODE_TILED", "0") == "1"   # decode GEMMs stream a tile-major weight copy (+13 GB)
-        self._wt: Dict[str, torch.Tensor] = {}
-        self.use_2cta = True           # cta_group::2 GEMM for the large prefill projections and 3x3 convs
-        self.fused_head_tail = os.environ.get("GROMA_FUSED_HEAD_TAIL", "1") != "0"   # decode: head reduce + argmax + advance in one launch
-        self.use_fused_rope = os.environ.get("GROMA_FUSED_ROPE", "1") != "0"   # RoPE + KV append in the qkv GEMM epilogue (prefill)
-        self.fuse_gn_apply = os.environ.get("GROMA_FUSE_GN", "1") != "0"       # GroupNorm + ReLU of a fusion round applied by the next round's shuffle
-        # tcgen05 flash attention (attention_tcgen05.cu: two query tiles in ping-pong, P in tensor memory) for head dims 64 / 128
-        # (DINOv2 and the LLaMA prefill); the mma.sync kernel stays for head dim 32 (Deformable-DETR self-attention) and the
-        # miniature test shapes.  GROMA_TC_ATTENTION=0 switches back for A/B runs.
-        self.use_tc_attention = os.environ.get("GROMA_TC_ATTENTION", "1") == "1"
-        self.use_megakernel = os.environ.get("GROMA_DECODE_MEGA", "0") == "1"   # one persistent kernel per decode step (csrc/decode_megakernel.cu)
+        # tests set these to False to run the reference arrangements
+        self.fuse_gn_apply = True    # GroupNorm + ReLU of a fusion round applied by the next round's shuffle
         self.fused_decode = True     # fused reduce epilogues + PDL in the decode step
-        self.fused_rope_attn = os.environ.get("GROMA_FUSED_ROPE_ATTN", "1") == "1"   # qkv reduce + RoPE + KV append inside the attention launch
         self.use_pdl = True
-        self.graph_proposer = os.environ.get("GROMA_GRAPH_PROPOSER", "1") == "1"
         self._prop_graphs: Dict[tuple, tuple] = {}
         self.topk_override = None  # tests: int64 [B, num_queries] token indices replacing the proposer's own top-k
-        self.timing_hook = None   # bench.py: list collecting (start_event, end_event, algorithmic_bytes) per swap-AB GEMM
 
     # ------------------------------------------------------------------------------------------ weights
     def _mat(self, t: torch.Tensor) -> torch.Tensor:
@@ -158,8 +146,8 @@ class GromaEngine:
         n_mid, ro = fw.shape[0], cfg.roi_out
         w["flatten.w"] = self._mat(fw.reshape(n_mid, H, ro * ro).permute(0, 2, 1).reshape(n_mid, ro * ro * H))  # (c,h,w) -> (h,w,c)
         w["flatten.b"] = self._vec(sd[re_ + "roi_align.flatten_linear.bias"])
-        # LLaMA.  The projections live in two arenas so that the persistent decode kernel addresses every weight tile through one
-        # TMA descriptor each (include/groma_b200.h: groma_decode_step_args); the per-layer entries of `w` are row views into them
+        # LLaMA.  The projections live in two arenas (qkv / o / gate-up of every layer + both heads, and the down projections);
+        # the per-layer entries of `w` are row views into them
         w["embed"] = self._mat(sd["llm.model.embed_tokens.weight"])
         w["new_embed"] = self._mat(sd["new_input_embs.weight"])
         L, I, V = cfg.llm_layers, cfg.llm_inter, cfg.vocab + cfg.num_new_token
@@ -272,7 +260,8 @@ class GromaEngine:
             o = f"vit.{i}."
             y = G.layernorm(x, w[o + "ln1.w"], w[o + "ln1.b"], cfg.vit_ln_eps)
             qkv = G.gemm(y, w[o + "qkv.w"], bias=w[o + "qkv.b"]).reshape(B, S, 3, nh, hd)
-            attn = G.attention_tc if (self.use_tc_attention and hd in (64, 128)) else G.attention
+            # tcgen05 flash attention for head dims 64 / 128; the mma.sync kernel for the others (the miniature test shapes)
+            attn = G.attention_tc if hd in (64, 128) else G.attention
             a = attn(qkv[:, :, 0], qkv[:, :, 1].permute(0, 2, 1, 3), qkv[:, :, 2].permute(0, 2, 1, 3),
                      causal=False, scale=1.0 / math.sqrt(hd))
             xn = torch.empty_like(x) if i >= keep_from else x   # keep the hidden states that are read later intact
@@ -310,7 +299,7 @@ class GromaEngine:
         valid until the next proposer() call of the same shape.  Parity runs that record stages / teacher-force the top-k go eager."""
         cfg = self.cfg
         B = hs[0].shape[0]
-        if not self.graph_proposer or self.keep_stages or self.topk_override is not None or torch.cuda.is_current_stream_capturing():
+        if self.keep_stages or self.topk_override is not None or torch.cuda.is_current_stream_capturing():
             x = G.mean_tokens(hs[-4:], 1).reshape(B * cfg.grid * cfg.grid, -1)
             return self._proposer_body(x, B, n_extra)
         key = (B, n_extra)
@@ -502,7 +491,7 @@ class GromaEngine:
             xs.append(G.gemm(up.reshape(-1, self.in_ld), w[f"inconv.{l}.w"], bias=w[f"inconv.{l}.b"]).reshape(B, s, s, C))
         # Between fusion rounds the maps stay RAW conv outputs + GroupNorm statistics: the next round's shuffle applies norm + ReLU
         # tap by tap (bit-identical to apply -> store -> shuffle, tests/test_ops_gpu.py), which drops one read + one write of every
-        # map per round; only the last round's maps are materialised for RoIAlign.  GROMA_FUSE_GN=0: the three-kernel form.
+        # map per round; only the last round's maps are materialised for RoIAlign.  fuse_gn_apply = False: the three-kernel form.
         st = None                                       # per-level statistics of the maps in xs (None = xs is already activated)
         for k in range(cfg.fuse_rounds):
             new, new_st = [], []
@@ -515,7 +504,7 @@ class GromaEngine:
                 else:
                     xin = G.fuse_shuffle_gn(xs[l], xs[t], xs[d], st[l], st[t], st[d], w[f"fuse.{k - 1}.gn.w"], w[f"fuse.{k - 1}.gn.b"],
                                             cfg.gn_groups)
-                y = G.conv3x3_flat(xin.reshape(-1, C), w[f"fuse.{k}.w"], B, s + 2, s + 2, block_n=512 if (self.use_2cta and C >= 512) else 0)
+                y = G.conv3x3_flat(xin.reshape(-1, C), w[f"fuse.{k}.w"], B, s + 2, s + 2, block_n=512 if C >= 512 else 0)
                 if self.fuse_gn_apply and not last:
                     new_st.append(G.groupnorm_stats(y, cfg.gn_groups, 1e-5, B))
                     new.append(y.reshape(B, s, s, C))
@@ -543,7 +532,7 @@ class GromaEngine:
         for l in range(3):
             G.roi_align(xs[l], rois, ro, (8, 4, 2)[l] / 14.0, cfg.roi_sampling, True, pad=True, out=rbuf[l])
         fused = G.conv3x3_flat(rbuf.reshape(-1, C), w["pconv.w"], K, rp, rp, bias=w["pconv.b"], act=G.ACT_RELU,
-                               block_n=512 if (self.use_2cta and C >= 512 and K * rp * rp >= 2048) else 0)  # [K*ro*ro, C]
+                               block_n=512 if (C >= 512 and K * rp * rp >= 2048) else 0)  # [K*ro*ro, C]
         self._stage("roi_fused", fused.reshape(K, ro, ro, C))
         flat_in = fused.reshape(K, ro * ro * C)
         kt = flat_in.shape[1]
@@ -593,10 +582,10 @@ class GromaEngine:
         q = torch.empty((B * T, nh * hd), dtype=torch.bfloat16, device=self.dev)
         # cta_group::2 (256x256 tiles per CTA pair) for the big projections: +4..8 % over the single-CTA tile; the 22016-wide
         # gate/up projection measured 3 % slower with it and keeps the 128x256 tile
-        bn2 = 512 if (self.use_2cta and B * T >= 2048 and cfg.llm_hidden >= 2048) else 0
+        bn2 = 512 if (B * T >= 2048 and cfg.llm_hidden >= 2048) else 0
         # RoPE + KV append in the qkv GEMM epilogue (one launch, no [B*T, 3*hidden] intermediate) whenever the 256-wide tile
         # applies: head_dim 128 and enough rows to fill the SMs; tiny test configs keep gemm + rope_kv (same values)
-        fused_rope = self.use_fused_rope and hd == 128 and nh % 2 == 0 and (bn2 == 512 or B * T >= 1024)
+        fused_rope = hd == 128 and nh % 2 == 0 and (bn2 == 512 or B * T >= 1024)
         for i in range(cfg.llm_layers):
             o = f"llm.{i}."
             y = G.rmsnorm(x, w[o + "ln1"], cfg.rms_eps)
@@ -606,7 +595,7 @@ class GromaEngine:
             else:
                 qkv = G.gemm(y, w[o + "qkv.w"], block_n=bn2)
                 G.rope_kv(qkv, q, kc, vc, self.rope_cos, self.rope_sin, B, T, nh, hd, 0)
-            attn = G.attention_tc if (self.use_tc_attention and hd in (64, 128)) else G.attention
+            attn = G.attention_tc if hd in (64, 128) else G.attention
             a = attn(q.reshape(B, T, nh, hd), kc, vc, causal=True, scale=1.0 / math.sqrt(hd), kv_len=kv_len, sk=T)
             G.gemm(a.reshape(B * T, nh * hd), w[o + "o.w"], residual=x, out=x, block_n=bn2)
             y = G.rmsnorm(x, w[o + "ln2"], cfg.rms_eps)
@@ -641,88 +630,9 @@ class GromaEngine:
             ws=torch.empty((16 * max(3 * Hd, 2 * I, V) * B,), dtype=torch.float32, device=self.dev),
             logits=torch.empty((B, V), dtype=torch.float32, device=self.dev),
             pos=torch.zeros((1,), dtype=torch.int32, device=self.dev),
-            cnt=torch.zeros((1024,), dtype=torch.int32, device=self.dev),   # split-K tile counters (self re-arming)
             kv_len=torch.zeros((B,), dtype=torch.int32, device=self.dev),
         )
         return d
-
-    # ------------------------------------------------------------------------------------------ persistent decode step
-    def mega_supported(self, B: int) -> bool:
-        cfg = self.cfg
-        return (cfg.head_dim == 128 and B <= 16 and cfg.llm_hidden % 128 == 0 and cfg.llm_inter % 64 == 0 and
-                (2 * cfg.llm_inter) % 128 == 0 and cfg.llm_hidden <= 8192)
-
-    def _mega_state(self, B: int):
-        """Scratch + argument block of groma_decode_step_fused for batch B (allocated once per B)."""
-        st = getattr(self, "_mk", None)
-        if st is not None and st["B"] == B:
-            return st
-        cfg = self.cfg
-        L, H, Hd, I, V = cfg.llm_layers, cfg.llm_heads, cfg.llm_hidden, cfg.llm_inter, cfg.vocab + cfg.num_new_token
-        n_flags, ws_tile, part, _ = G.decode_step_layout(L, B, H, Hd, I, V)
-        sms = torch.cuda.get_device_properties(self.dev).multi_processor_count
-        # every CTA needs at least one (row tile, k-block) unit of every projection (contributors of a tile are consecutive CTAs)
-        units = min(3 * Hd // 128 * (Hd // 64), Hd // 128 * (Hd // 64), 2 * I // 128 * (Hd // 64), Hd // 128 * (I // 64), (V + 127) // 128 * (Hd // 64))
-        grid = max(1, min(sms, units, int(os.environ.get("GROMA_MEGA_GRID", "100000"))))
-        s_att = max(1, min(32, -(-int(os.environ.get("GROMA_MEGA_ITEMS_PER_CTA", "4")) * grid // (B * H))))
-        f32 = lambda n: torch.empty((n,), dtype=torch.float32, device=self.dev)
-        with torch.inference_mode(False):
-            st = dict(B=B, grid=grid, s_att=s_att,
-                      y2=torch.empty((B, Hd), dtype=torch.bfloat16, device=self.dev),
-                      ws_qkv=f32(3 * Hd // 128 * ws_tile), ws_o=f32(Hd // 128 * ws_tile), ws_gu=f32(2 * I // 128 * ws_tile),
-                      ws_down=f32(Hd // 128 * ws_tile), ws_head=f32((V + 127) // 128 * ws_tile),
-                      att_part=f32(B * H * s_att * part), cand_val=f32((V + 127) // 128 * 16),
-                      cand_idx=torch.empty(((V + 127) // 128 * 16,), dtype=torch.int32, device=self.dev),
-                      flags=torch.zeros((n_flags,), dtype=torch.int32, device=self.dev),
-                      status=torch.zeros((8 + 16 * sms,), dtype=torch.int32, device=self.dev), timeline=None)
-        self._mk = st
-        return st
-
-    def decode_step_mega(self, B: int) -> torch.Tensor:
-        """The same greedy step as decode_step() in ONE persistent kernel (csrc/decode_megakernel.cu): reads d['ids'], *pos,
-        kv_len; appends K/V; writes d['logits'], the next ids, and advances pos / kv_len.  CUDA-graph capturable (the flag
-        reset is a fill on the same stream)."""
-        cfg, w = self.cfg, self.w
-        d = self._decode_buffers(B)
-        st = self._mega_state(B)
-        a = G.DecodeStepArgs()
-        a.L, a.B, a.H, a.Hd, a.I, a.V = cfg.llm_layers, B, cfg.llm_heads, cfg.llm_hidden, cfg.llm_inter, cfg.vocab + cfg.num_new_token
-        a.vocab, a.S_att, a.cap = cfg.vocab, st["s_att"], self.kv_cap
-        a.scale, a.eps = 1.0 / math.sqrt(cfg.head_dim), cfg.rms_eps
-        ptr = lambda t: t.data_ptr()
-        a.w_arena, a.w_down, a.embed, a.new_embed, a.ln_w = ptr(self.llm_arena), ptr(self.llm_down), ptr(w["embed"]), ptr(w["new_embed"]), ptr(self.llm_ln)
-        a.kv, a.rope_cos, a.rope_sin = ptr(self.kv), ptr(self.rope_cos), ptr(self.rope_sin)
-        a.ids, a.pos, a.kv_len = ptr(d["ids"]), ptr(d["pos"]), ptr(d["kv_len"])
-        a.x, a.y_attn, a.y_mlp, a.a, a.gu, a.logits = ptr(d["x"]), ptr(d["y"]), ptr(st["y2"]), ptr(d["a"]), ptr(d["gu"]), ptr(d["logits"])
-        for k in ("ws_qkv", "ws_o", "ws_gu", "ws_down", "ws_head", "att_part", "cand_val", "cand_idx", "flags", "status"):
-            setattr(a, k, ptr(st[k]))
-        a.grid = st["grid"]
-        a.l2_prefetch_slots = int(os.environ.get("GROMA_MEGA_PREFETCH", "0"))
-        a.timeline = st["timeline"].data_ptr() if st["timeline"] is not None else None
-        if tuple(self.kv.shape[2:4]) != (B, cfg.llm_heads):
-            raise RuntimeError("KV cache was allocated for a different batch")
-        st["flags"].zero_()
-        G.decode_step_fused(a)
-        return d["logits"]
-
-    def check_decode_status(self):
-        """Raise if a dependency wait of the persistent decode kernel timed out (one device->host read; call outside graphs)."""
-        st = getattr(self, "_mk", None)
-        if st is None:
-            return
-        s = st["status"].cpu().tolist()
-        if s[0] != 0:
-            st["status"].zero_()
-            from collections import Counter
-            roles = ("stream-loader", "mma", "worker", "activation-loader")
-            parked = Counter((roles[r], s[8 + (c * 4 + r) * 4], s[8 + (c * 4 + r) * 4 + 1] if os.environ.get("GROMA_MEGA_DEBUG") else 0)
-                             for c in range(st["grid"]) for r in range(4) if s[8 + (c * 4 + r) * 4] != 0)
-            detail = ""
-            if os.environ.get("GROMA_MEGA_DEBUG"):
-                detail = "\n" + "\n".join(f"cta {c} {roles[r]}: {s[8 + (c * 4 + r) * 4: 12 + (c * 4 + r) * 4]}" for c in range(st["grid"]) for r in range(4)
-                                          if s[8 + (c * 4 + r) * 4] != 0)
-            raise G._lib.GromaError(f"persistent decode kernel aborted: code {s[0]} (cta {s[1]}, role {roles[s[2]]}, thread {s[3]}, info {s[4:7]}); "
-                                    f"parked waits (role, code, info): {sorted(parked.items(), key=lambda kv: -kv[1])[:12]}{detail}")
 
     def _decode_splits(self):
         """Split-K factors of the five decode GEMMs: (weight row-tiles of 128) x split should fill whole waves of the 296
@@ -730,8 +640,7 @@ class GromaEngine:
         2.9 waves."""
         if getattr(self, "_splits", None) is None:
             cfg = self.cfg
-
-            ncta = 148 * max(1, int(os.environ.get("GROMA_GEMM_CTAS_PER_SM", "2")))   # the BN=16 kernel runs 2 CTAs per SM
+            ncta = 148 * 2   # launch_gemm in csrc/gemm.cu runs the BN=16 kernel 2 CTAs per SM: change both together
 
             def pick(n_rows, k):
                 tiles = (n_rows + 127) // 128
@@ -757,29 +666,10 @@ class GromaEngine:
         W = self.w[wname]
         N, B = W.shape[0], x.shape[0]
         ws = d["ws"][: split * N * B].view(split, N, B)
-        if self.timing_hook is not None:
-            ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            ev0.record()
-        if self.fused_splitk:
-            # one launch: the CTA finishing a tile last reduces the partials (measured SLOWER at decode tile sizes: the
-            # per-tile release fence + atomic sit on the epilogue's critical path; kept for larger-K uses, off by default)
-            G.gemm_swap_ab_fused(x, W, ws, d["cnt"], split, out, act=act, residual=residual)
-        else:
-            G.gemm_swap_ab(x, W, ws, split_k=split)
-        if self.timing_hook is not None:
-            ev1.record()
-            self.timing_hook.append((ev0, ev1, W.numel() * 2 + x.numel() * 2 + ws.numel() * 4))
-        if not self.fused_splitk:
-            n_out = N // 2 if act == G.ACT_SWIGLU else N
-            G.splitk_reduce(ws, out, act=act, residual=residual, bias_along_m=True, ld_m=1, ld_n=n_out)
+        G.gemm_swap_ab(x, W, ws, split_k=split)
+        n_out = N // 2 if act == G.ACT_SWIGLU else N
+        G.splitk_reduce(ws, out, act=act, residual=residual, bias_along_m=True, ld_m=1, ld_n=n_out)
         return out
-
-    def _tiled(self, wname: str) -> torch.Tensor:
-        """Tile-major copy of a decode weight (every 128x64 TMA box = one contiguous 16 KB run of HBM); built on first use."""
-        t = self._wt.get(wname)
-        if t is None:
-            t = self._wt[wname] = G.tile_weight(self.w[wname])
-        return t
 
     def decode_step(self, B: int) -> torch.Tensor:
         """One greedy decode step for the whole batch (groma.py:376-402 + HF greedy argmax): reads d['ids'], appends K/V at
@@ -787,8 +677,6 @@ class GromaEngine:
         Every shape-dependent scalar lives on the device, so the step is CUDA-graph capturable.
         Per layer: 4 swap-AB tcgen05 GEMMs (weights prefetched under programmatic dependent launch), 4 fused reduce
         epilogues (RoPE+KV append / residual+RMSNorm / SwiGLU / residual+next RMSNorm) and the cluster decode attention."""
-        if self.use_megakernel and self.mega_supported(B):
-            return self.decode_step_mega(B)
         if not self.fused_decode:
             return self._decode_step_unfused(B)
         cfg, w = self.cfg, self.w
@@ -803,31 +691,19 @@ class GromaEngine:
         def gemm(inp, wname, split):
             W = w[wname]
             ws = d["ws"][: split * W.shape[0] * B].view(split, B, W.shape[0])
-            if self.timing_hook is not None:
-                ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                ev0.record()
-            if self.decode_tiled:
-                G.gemm_swap_ab(inp, self._tiled(wname), ws, split_k=split, pdl=pdl, transposed=True, tiled=True, n_rows=W.shape[0])
-            else:
-                G.gemm_swap_ab(inp, W, ws, split_k=split, pdl=pdl, transposed=True)
-            if self.timing_hook is not None:
-                ev1.record()
-                self.timing_hook.append((ev0, ev1, W.numel() * 2 + inp.numel() * 2 + ws.numel() * 4))
+            G.gemm_swap_ab(inp, W, ws, split_k=split, pdl=pdl, transposed=True)
             return ws
 
         for i in range(cfg.llm_layers):
             o = f"llm.{i}."
             kc, vc = self.kv[i, 0], self.kv[i, 1]
             ws = gemm(y, o + "qkv.w", sp["qkv"])
-            if hd == 128 and self.fused_rope_attn:
+            if hd == 128:   # qkv reduce + RoPE + KV append inside the attention launch
                 G.decode_rope_attention(ws, kc, vc, d["kv_len"], d["pos"], self.rope_cos, self.rope_sin, 1.0 / math.sqrt(hd), d["a"], pdl=pdl)
             else:
                 G.decode_reduce_rope_kv(ws, d["q"], kc, vc, self.rope_cos, self.rope_sin, d["pos"], nh, hd, pdl=pdl)
-                if hd == 128:
-                    G.decode_attention(d["q"], kc, vc, d["kv_len"], 1.0 / math.sqrt(hd), d["a"], pdl=pdl)
-                else:
-                    G.attention(d["q"].reshape(B, 1, nh, hd), kc, vc, causal=False, scale=1.0 / math.sqrt(hd), kv_len=d["kv_len"],
-                                out=d["a"], sk=self.kv_cap)
+                G.attention(d["q"].reshape(B, 1, nh, hd), kc, vc, causal=False, scale=1.0 / math.sqrt(hd), kv_len=d["kv_len"],
+                            out=d["a"], sk=self.kv_cap)
             ws = gemm(d["a"].reshape(B, Hd), o + "o.w", sp["o"])
             G.decode_reduce_norm(ws, x, w[o + "ln2"], y, cfg.rms_eps, pdl=pdl)
             ws = gemm(y, o + "gu.w", sp["gu"])
@@ -836,12 +712,7 @@ class GromaEngine:
             nxt = w[f"llm.{i + 1}.ln1"] if i + 1 < cfg.llm_layers else w["llm.norm"]
             G.decode_reduce_norm(ws, x, nxt, y, cfg.rms_eps, pdl=pdl)
         ws = gemm(y, "head.w", sp["head"])
-        if self.fused_head_tail:
-            G.decode_head_argmax(ws, d["logits"], d["ids"], d["pos"], d["kv_len"], pdl=pdl)   # reduce + argmax + advance, one launch
-        else:
-            G.splitk_reduce(ws, d["logits"])
-            G.argmax(d["logits"], out=d["ids"])
-            G.decode_advance(d["pos"], d["kv_len"])
+        G.decode_head_argmax(ws, d["logits"], d["ids"], d["pos"], d["kv_len"], pdl=pdl)   # reduce + argmax + advance, one launch
         return d["logits"]
 
     def _decode_step_unfused(self, B: int) -> torch.Tensor:

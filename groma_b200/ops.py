@@ -70,7 +70,7 @@ def gemm(a: torch.Tensor, w: torch.Tensor, *, bias: Optional[torch.Tensor] = Non
         _bf16(residual, "residual")
         assert residual.stride() == out.stride()
     rc = _L().groma_gemm_bf16(_p(a), a.shape[0], a.stride(0), _p(w), w.shape[0], w.stride(0), M, N, K, 1, None,
-                              _p(out), out.stride(0), 1, flags, act, _p(bias), _p(gamma), _p(residual), None, 1, None, 0, 0,
+                              _p(out), out.stride(0), 1, flags, act, _p(bias), _p(gamma), _p(residual), None, 1, 0, 0,
                               block_n, _stream())
     _chk(rc, "groma_gemm_bf16")
     return out
@@ -101,7 +101,7 @@ def gemm_splitk(a: torch.Tensor, w: torch.Tensor, split_k: int, *, bias=None, ac
     if ws is None:
         ws = torch.empty((split_k, M, N), dtype=torch.float32, device=a.device)
     rc = _L().groma_gemm_bf16(_p(a), M, a.stride(0), _p(w), N, w.stride(0), M, N, K, 1, None, None, 0, 0, GF_PARTIAL,
-                              ACT_NONE, None, None, None, _p(ws), split_k, None, 0, 0, block_n, _stream())
+                              ACT_NONE, None, None, None, _p(ws), split_k, 0, 0, block_n, _stream())
     _chk(rc, "groma_gemm_bf16(split-k)")
     n_out = N // 2 if act == ACT_SWIGLU else N
     if out is None:
@@ -113,50 +113,22 @@ def gemm_splitk(a: torch.Tensor, w: torch.Tensor, split_k: int, *, bias=None, ac
     return out
 
 
-GF_A_TILED, GF_PDL, GF_PARTIAL_T = 32, 64, 128
-
-
-def tile_weight(w: torch.Tensor) -> torch.Tensor:
-    """[N, K] -> tile-major [(N/128)*(K/64)*128, 64] (zero padded): every 128x64 TMA tile is one contiguous 16 KB."""
-    N, K = w.shape
-    Np, Kp = (N + 127) // 128 * 128, (K + 63) // 64 * 64
-    if (Np, Kp) != (N, K):
-        wp = torch.zeros((Np, Kp), dtype=w.dtype, device=w.device)
-        wp[:N, :K] = w
-        w = wp
-    return w.view(Np // 128, 128, Kp // 64, 64).permute(0, 2, 1, 3).contiguous().view(-1, 64)
+GF_PDL, GF_PARTIAL_T = 64, 128
 
 
 def gemm_swap_ab(x: torch.Tensor, w: torch.Tensor, ws: torch.Tensor, split_k: int = 1, block_n: int = 0,
-                 n_rows: Optional[int] = None, tiled: bool = False, pdl: bool = False, transposed: bool = False) -> torch.Tensor:
+                 pdl: bool = False, transposed: bool = False) -> torch.Tensor:
     """Skinny-M GEMM for decode: computes (w[N,K] @ x[M,K]^T) with the weight as the 128-row MMA operand and the
     M<=256 activation rows as the MMA N dimension; raw fp32 partials land in ws[split][N][M].
-    tiled: w is the output of tile_weight() (then n_rows = logical N).  pdl: programmatic dependent launch."""
-    _bf16(x, "x"); _bf16(w, "w")
-    M, K = x.shape
-    N = w.shape[0] if n_rows is None else n_rows
-    flags = GF_PARTIAL | (GF_A_TILED if tiled else 0) | (GF_PDL if pdl else 0) | (GF_PARTIAL_T if transposed else 0)
-    rc = _L().groma_gemm_bf16(_p(w), w.shape[0], w.stride(0), _p(x), M, x.stride(0), N, M, K, 1, None, None, 0, 0, flags,
-                              ACT_NONE, None, None, None, _p(ws), split_k, None, 0, 0, block_n, _stream())
-    _chk(rc, "groma_gemm_bf16(swap-ab)")
-    return ws
-
-
-def gemm_swap_ab_fused(x: torch.Tensor, w: torch.Tensor, ws: torch.Tensor, counters: torch.Tensor, split_k: int,
-                       out: torch.Tensor, *, act: int = ACT_NONE, residual: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """Decode GEMM in one launch: out[M, N(/2)] = epilogue(x[M,K] @ w[N,K]^T).  Weights are the 128-row MMA operand
-    (swap-AB), K is split over CTAs, and the CTA that finishes a weight tile last reduces the fp32 partials and writes the
-    bf16 / fp32 rows of `out` (transposed store, optional residual add, optional SwiGLU over interleaved weight rows)."""
+    pdl: programmatic dependent launch."""
     _bf16(x, "x"); _bf16(w, "w")
     M, K = x.shape
     N = w.shape[0]
-    n_out = N // 2 if act == ACT_SWIGLU else N
-    assert out.shape == (M, n_out) and out.is_contiguous() and counters.dtype == torch.int32
-    flags = GF_PARTIAL | GF_BIAS_ALONG_M | (GF_OUT_F32 if out.dtype == torch.float32 else 0)
-    rc = _L().groma_gemm_bf16(_p(w), N, w.stride(0), _p(x), M, x.stride(0), N, M, K, 1, None, _p(out), 1, n_out, flags, act,
-                              None, None, _p(residual), _p(ws), split_k, _p(counters), 0, 0, 0, _stream())
-    _chk(rc, "groma_gemm_bf16(swap-ab fused)")
-    return out
+    flags = GF_PARTIAL | (GF_PDL if pdl else 0) | (GF_PARTIAL_T if transposed else 0)
+    rc = _L().groma_gemm_bf16(_p(w), N, w.stride(0), _p(x), M, x.stride(0), N, M, K, 1, None, None, 0, 0, flags,
+                              ACT_NONE, None, None, None, _p(ws), split_k, 0, 0, block_n, _stream())
+    _chk(rc, "groma_gemm_bf16(swap-ab)")
+    return ws
 
 
 def conv3x3_flat(x_pad: torch.Tensor, w_taps: torch.Tensor, n_img: int, hp: int, wp: int, *, bias=None, act=ACT_NONE,
@@ -184,7 +156,7 @@ def conv3x3_flat(x_pad: torch.Tensor, w_taps: torch.Tensor, n_img: int, hp: int,
     flags = GF_CONV_ROWS | (GF_CONV_COMPACT if compact else 0)
     rc = _L().groma_gemm_bf16(_p(x_pad), x_pad.shape[0], x_pad.stride(0), _p(w_taps), Cout, w_taps.stride(0), rows,
                               Cout, C, L * 9, _i32_array(offs), _p(out), out.stride(0), 1, flags, act, _p(bias), None,
-                              None, None, 1, None, hp, wp, block_n, _stream())
+                              None, None, 1, hp, wp, block_n, _stream())
     _chk(rc, "groma_gemm_bf16(conv3x3)")
     return out
 
@@ -608,29 +580,6 @@ def decode_rope_attention(ws: torch.Tensor, cache_k: torch.Tensor, cache_v: torc
     _chk(_L().groma_decode_rope_attention(_p(ws), S, _p(cache_k), _p(cache_v), _p(out), _p(kv_len), _p(pos_ptr), _p(cos_t), _p(sin_t),
                                           B, H, D, cap, float(scale), 1 if pdl else 0, _stream()), "groma_decode_rope_attention")
     return out
-
-
-# --------------------------------------------------------------------------------------------- persistent decode step
-class DecodeStepArgs(ctypes.Structure):
-    """`groma_decode_step_args` of include/groma_b200.h, field for field."""
-    _fields_ = ([(n, ctypes.c_int32) for n in ("L", "B", "H", "Hd", "I", "V", "vocab", "S_att")] + [("cap", ctypes.c_int64)] +
-                [("scale", ctypes.c_float), ("eps", ctypes.c_float)] +
-                [(n, ctypes.c_void_p) for n in ("w_arena", "w_down", "embed", "new_embed", "ln_w", "kv", "rope_cos", "rope_sin", "ids", "pos",
-                                                "kv_len", "x", "y_attn", "y_mlp", "a", "gu", "logits", "ws_qkv", "ws_o", "ws_gu", "ws_down",
-                                                "ws_head", "att_part", "cand_val", "cand_idx", "flags", "status")] +
-                [("grid", ctypes.c_int32), ("l2_prefetch_slots", ctypes.c_int32), ("timeline", ctypes.c_void_p)])
-
-
-def decode_step_layout(L: int, B: int, H: int, Hd: int, I: int, V: int):
-    """(number of int32 flags, fp32 scratch floats per 128-row weight tile, floats per attention partial, max rows)."""
-    out = (ctypes.c_int64 * 4)()
-    _lib.check(_L().groma_decode_step_layout(L, B, H, Hd, I, V, ctypes.cast(out, ctypes.c_void_p), None), "groma_decode_step_layout")
-    return [int(v) for v in out]
-
-
-def decode_step_fused(args: DecodeStepArgs) -> None:
-    """One persistent-kernel decode step (all layers + heads + argmax); `flags` must have been zeroed on the same stream."""
-    _chk(_L().groma_decode_step_fused(ctypes.cast(ctypes.pointer(args), ctypes.c_void_p), _stream()), "groma_decode_step_fused")
 
 
 # ----------------------------------------------------------------------------------------------------------------------

@@ -36,7 +36,6 @@ extern "C" {
 #define GROMA_GF_PARTIAL 4
 #define GROMA_GF_CONV_ROWS 8
 #define GROMA_GF_CONV_COMPACT 16
-#define GROMA_GF_A_TILED 32 /* A pre-tiled [m_tile][k_block][128][64] (lda must be 64): each TMA load is 16 KB contiguous */
 #define GROMA_GF_PARTIAL_T 128 /* partials transposed: ws[split][n][m] */
 #define GROMA_GF_PDL 64     /* programmatic dependent launch: A tiles are prefetched before waiting for the previous kernel */
 
@@ -50,15 +49,12 @@ extern "C" {
  * residual bf16 with the strides of out.  GROMA_GF_PARTIAL: raw fp32 accumulators to ws[split][M][N] (split_k >= 1).
  * GROMA_GF_CONV_ROWS: rows are pixels of [img][conv_hp][conv_wp] maps, border rows are not written;
  * with GROMA_GF_CONV_COMPACT the row index is that of the un-padded [img][hp-2][wp-2] layout.
- * tile_counters (optional, with GROMA_GF_PARTIAL): zero-initialised int32[m_tiles*n_tiles]; the CTA that delivers the last
- * split of a tile sums ws over the splits in fixed order and applies the epilogue to `out` itself (no groma_splitk_reduce
- * launch); with GROMA_ACT_SWIGLU + GROMA_GF_BIAS_ALONG_M the (gate, up) pairs are adjacent ROWS (swap-AB decode layout).
  * block_n: 0 = auto, else 16/32/64/128/256. */
 int32_t groma_gemm_bf16(const void* A, int64_t a_rows, int64_t lda, const void* B, int64_t b_rows, int64_t ldb,
                         int32_t M, int32_t N, int32_t K, int32_t num_taps, const int32_t* a_row_off /*host*/,
                         void* out, int64_t ld_m, int64_t ld_n, int32_t flags, int32_t act, const float* bias,
                         const float* gamma, const void* residual, float* ws, int32_t split_k,
-                        int32_t* tile_counters, int32_t conv_hp, int32_t conv_wp, int32_t block_n, void* stream);
+                        int32_t conv_hp, int32_t conv_wp, int32_t block_n, void* stream);
 
 /* LLaMA attention input in ONE launch: x[B*T, K] @ w_qkv[3*H*D, K]^T (rows of w_qkv = [q heads | k heads | v heads]) with the
  * rotate-half RoPE of q and k and the KV-cache append done in the GEMM epilogue -- the [B*T, 3*H*D] intermediate of
@@ -233,53 +229,6 @@ int32_t groma_decode_head_argmax(const float* ws, int32_t splits, int32_t B, int
 int32_t groma_decode_reduce_rope_kv(const float* ws, int32_t splits, int32_t B, int32_t H, int32_t D, void* q_out, void* cache_k,
                                     void* cache_v, const float* cos_t, const float* sin_t, const int32_t* pos_ptr, int64_t cap,
                                     int32_t pdl, void* stream);
-
-/* ---- one persistent kernel per greedy decode step --------------------------------------------------------------------------
- * Replaces, for B <= 16 rows and head_dim 128, everything the reference executes per generated token: GromaModel.forward's
- * decode branch (groma/model/groma.py:376-402: embedding of the last id, 32 x LlamaDecoderLayer with KV append
- * -- $HF/models/llama/modeling_llama.py:292-340 -- final norm, lm_head || extra_lm_head) and the argmax of HF greedy search.
- * One launch of one CTA per SM; the weight / KV stream of each CTA is a single in-order ring filled by TMA that never waits for
- * activations (groma_b200/csrc/decode_megakernel.cu).  All pointers are device pointers owned by the caller:
- *   w_arena  [L*(3Hd + Hd + 2I) + V, Hd] bf16: per layer q|k|v rows, o rows, (gate_j, up_j)-interleaved rows; then lm_head || extra_lm_head
- *   w_down   [L*Hd, I] bf16;  ln_w [2L+1][Hd] fp32: input_layernorm_l, post_attention_layernorm_l (l = 0..L-1), final norm
- *   kv       [L][2][B][H][cap][128] bf16 cache; rope_cos/sin [>= pos+1][64] fp32
- *   ids [B] int64 (in: token to embed; out: next greedy token), pos [1], kv_len [B] (advanced by the kernel)
- *   x, y_attn, y_mlp, a [B][Hd] bf16, gu [B][I] bf16, logits [B][V] fp32 (written), ws_* fp32 scratch of
- *   tiles * layout[1] floats (tiles = rows/128 of the projection), att_part [B*H*S_att * layout[2]] floats,
- *   cand_val / cand_idx [ceil(V/128) * 16], flags int32[layout[0]] -- MUST be zero at entry (cudaMemsetAsync / fill before
- *   every step), status int32[8 + 16 * grid] -- zero at allocation; status[0] != 0 after the step = a dependency wait timed out
- *   (status[1..6]: CTA, role, thread, progress counters; from [8]: per (CTA, role) the wait it was parked in) and the outputs
- *   are invalid.
- * S_att: key segments per (row, head), merged in fixed order; choose it so that B*H*S_att is a few times the SM count.
- * grid: 0 = one CTA per SM (must not exceed the SM count: all CTAs have to be co-resident). */
-typedef struct groma_decode_step_args {
-    int32_t L, B, H, Hd, I, V, vocab, S_att;
-    int64_t cap;
-    float scale, eps;
-    const void *w_arena, *w_down, *embed, *new_embed;
-    const float* ln_w;
-    void* kv;
-    const float *rope_cos, *rope_sin;
-    int64_t* ids;
-    int32_t* pos;
-    int32_t* kv_len;
-    void *x, *y_attn, *y_mlp, *a, *gu;
-    float* logits;
-    float *ws_qkv, *ws_o, *ws_gu, *ws_down, *ws_head;
-    float* att_part;
-    float* cand_val;
-    int32_t* cand_idx;
-    int32_t* flags;
-    int32_t* status;
-    int32_t grid;
-    int32_t l2_prefetch_slots; /* 16 KB slots the L2 prefetcher keeps ahead of the shared-memory ring (0 = no prefetch) */
-    int64_t* timeline;   /* optional (may be null): int64[grid*4*32] %globaltimer stamps of the phase boundaries, for profiling */
-} groma_decode_step_args;
-int32_t groma_decode_step_fused(const groma_decode_step_args* args /*host*/, void* stream);
-/* layout[0] = number of int32 dependency flags, [1] = fp32 scratch floats per 128-row weight tile, [2] = floats per attention
- * partial, [3] = max rows per step (host array of 4). */
-int32_t groma_decode_step_layout(int32_t L, int32_t B, int32_t H, int32_t Hd, int32_t I, int32_t V, int64_t* layout /*host*/,
-                                 void* stream);
 
 /* greedy next-token argmax over fp32 logits (HF greedy_search). */
 int32_t groma_argmax(const float* logits, int64_t* out, int32_t rows, int32_t V, int64_t ld, void* stream);

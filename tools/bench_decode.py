@@ -47,18 +47,17 @@ torch.cuda.current_stream().wait_stream(s)
 us = timeit(lambda: g2.replay(), do_flush=False) / 64
 print(f"graph of 64 chained qkv swap-AB GEMMs (100 MB each): {us:.1f} us per launch = {3*Hd*Hd*2/us/1e3:.0f} GB/s")
 
-# ---- layout / launch variants of the decode GEMM inside a realistic chain (rmsnorm -> GEMM -> reduce), CUDA graph
+# ---- launch variants of the decode GEMM inside a realistic chain (rmsnorm -> GEMM -> reduce), CUDA graph
 big = torch.randn(1 << 28, device="cuda")
 print(f"torch.sum over 1 GiB fp32 (read-only stream): {big.numel()*4/timeit(lambda: big.sum(), iters=5)/1e3:.0f} GB/s")
 del big
-def chain(tiled, pdl, N, K, S, n=48):
-    ws_list = [torch.randn(N, K, device="cuda").bfloat16() for _ in range(8)]
-    wl = [G.tile_weight(w) for w in ws_list] if tiled else ws_list
+def chain(pdl, N, K, S, n=48):
+    wl = [torch.randn(N, K, device="cuda").bfloat16() for _ in range(8)]
     xx = torch.randn(B, K, device="cuda").bfloat16(); yy = torch.empty_like(xx); wn = torch.ones(K, device="cuda")
     wsb = torch.empty(S, N, B, device="cuda"); oo = torch.empty(B, N, device="cuda", dtype=torch.bfloat16)
     def body(i):
         G.rmsnorm(xx, wn, 1e-5, out=yy)
-        G.gemm_swap_ab(yy, wl[i % 8], wsb, split_k=S, n_rows=N, tiled=tiled, pdl=pdl)
+        G.gemm_swap_ab(yy, wl[i % 8], wsb, split_k=S, pdl=pdl)
         G.splitk_reduce(wsb, oo, bias_along_m=True, ld_m=1, ld_n=N)
     g = torch.cuda.CUDAGraph()
     st = torch.cuda.Stream(); st.wait_stream(torch.cuda.current_stream())
@@ -68,10 +67,9 @@ def chain(tiled, pdl, N, K, S, n=48):
             for i in range(n): body(i)
     torch.cuda.current_stream().wait_stream(st)
     us = timeit(lambda: g.replay(), do_flush=False) / n
-    ref = (yy.float() @ ws_list[(n - 1) % 8].float().t())
+    ref = (yy.float() @ wl[(n - 1) % 8].float().t())
     err = ((oo.float() - ref).abs().max() / ref.abs().max()).item()
-    print(f"chain N={N} K={K} S={S} tiled={int(tiled)} pdl={int(pdl)}: {us:.1f} us per (norm+gemm+reduce)  weights {N*K*2/us/1e3:.0f} GB/s  err {err:.1e}", flush=True)
+    print(f"chain N={N} K={K} S={S} pdl={int(pdl)}: {us:.1f} us per (norm+gemm+reduce)  weights {N*K*2/us/1e3:.0f} GB/s  err {err:.1e}", flush=True)
 for (N, K, S) in [(12288, 4096, 3), (22016, 4096, 6), (4096, 11008, 9), (4096, 4096, 13)]:
-    for tiled in (False, True):
-        for pdl in (False, True):
-            chain(tiled, pdl, N, K, S)
+    for pdl in (False, True):
+        chain(pdl, N, K, S)

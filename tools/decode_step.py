@@ -1,5 +1,5 @@
 """Time the real decode step (CUDA graph, Groma-7B LLaMA, B=16, ctx ~1030) and its GEMM-only / attention-only subsets.
-A/B knobs via env: GROMA_B200_LIB, GROMA_L2_PREFETCH, GROMA_GEMM_EARLY_TRIGGER, GROMA_DEC_UNROLL.
+A/B of builds via env: GROMA_B200_LIB.
     python tools/decode_step.py [ctx]"""
 import os, sys, math, torch
 sys.path.insert(0, ".")
@@ -53,10 +53,7 @@ sp = eng._decode_splits()
 def one(wn, s, src):
     W = eng.w[wn]
     ws = d["ws"][: s * W.shape[0] * B].view(s, B, W.shape[0])
-    if eng.decode_tiled:
-        G.gemm_swap_ab(d[src], eng._tiled(wn), ws, split_k=s, pdl=eng.use_pdl, transposed=True, tiled=True, n_rows=W.shape[0])
-    else:
-        G.gemm_swap_ab(d[src], W, ws, split_k=s, pdl=eng.use_pdl, transposed=True)
+    G.gemm_swap_ab(d[src], W, ws, split_k=s, pdl=eng.use_pdl, transposed=True)
 def gemms():
     for i in range(L):
         for wn, s, src in ((f"llm.{i}.qkv.w", sp["qkv"], "y"), (f"llm.{i}.o.w", sp["o"], "q"), (f"llm.{i}.gu.w", sp["gu"], "y"), (f"llm.{i}.down.w", sp["down"], "gu")):

@@ -1,6 +1,6 @@
 """Empirical split-K choice for the five swap-AB decode GEMM shapes (B=16): in-graph time of 24 back-to-back launches (PDL, weights
 rotating over copies larger than L2) per split factor.   python tools/sweep_decode_splits.py"""
-import os, sys, torch
+import sys, torch
 sys.path.insert(0, ".")
 from groma_b200 import ops as G
 
@@ -14,22 +14,19 @@ def timeit(fn, iters=20, warm=3):
 
 B = 16
 st = torch.cuda.Stream()
-tiled = os.environ.get("TILED", "0") == "1"
 shapes = dict(qkv=(12288, 4096), o=(4096, 4096), gu=(22016, 4096), down=(4096, 11008), head=(32114, 4096))
 only = sys.argv[1:] or list(shapes)
 for name in only:
     N, K = shapes[name]
     copies = max(2, int(300e6 // (N * K * 2)) + 1)
     wl = [torch.randn(N, K, device="cuda").bfloat16() for _ in range(copies)]
-    wt = [G.tile_weight(w) for w in wl] if tiled else None
     x = torch.randn(B, K, device="cuda").bfloat16()
     res = []
     for S in (1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12, 14, 16):
         if S > (K + 63) // 64: continue
         ws = torch.empty(S, B, N, device="cuda")
         def one(i):
-            if tiled: G.gemm_swap_ab(x, wt[i % copies], ws, split_k=S, pdl=True, transposed=True, tiled=True, n_rows=N)
-            else: G.gemm_swap_ab(x, wl[i % copies], ws, split_k=S, pdl=True, transposed=True)
+            G.gemm_swap_ab(x, wl[i % copies], ws, split_k=S, pdl=True, transposed=True)
         g = torch.cuda.CUDAGraph()
         st.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(st):
@@ -42,5 +39,5 @@ for name in only:
         print(f"{name:5s} N={N} K={K} S={S:2d}: {us:6.2f} us  {N * K * 2 / us / 1e3:5.0f} GB/s", flush=True)
     best = min(res)
     print(f"{name:5s} best split {best[1]} at {best[0]:.2f} us = {N * K * 2 / best[0] / 1e3:.0f} GB/s", flush=True)
-    del wl, wt
+    del wl
     torch.cuda.empty_cache()

@@ -1,5 +1,5 @@
-"""A/B of decode tunables on the B200: run as  GROMA_DEC_UNROLL=u [GROMA_B200_LIB=...] python tools/tune_decode.py"""
-import os, sys, math, torch
+"""A/B of the decode swap-AB GEMM across builds on the B200: run as  [GROMA_B200_LIB=...] python tools/tune_decode.py"""
+import os, sys, torch
 sys.path.insert(0, ".")
 from groma_b200 import ops as G
 def timeit(fn, iters=30, warm=5):
@@ -9,19 +9,8 @@ def timeit(fn, iters=30, warm=5):
         s = torch.cuda.Event(enable_timing=True); e = torch.cuda.Event(enable_timing=True)
         s.record(); fn(); e.record(); torch.cuda.synchronize(); ts.append(s.elapsed_time(e))
     ts.sort(); return ts[len(ts) // 2] * 1000
-B, H, D, cap = 16, 32, 128, 1100
-L = 6   # rotate over 6 layers of KV (>> L2)
-q = torch.randn(B, H * D, device="cuda").bfloat16(); out = torch.empty_like(q)
-kcs = [torch.randn(B, H, cap, D, device="cuda").bfloat16() for _ in range(L)]; vcs = [torch.randn(B, H, cap, D, device="cuda").bfloat16() for _ in range(L)]
-kvl = torch.full((B,), 1030, dtype=torch.int32, device="cuda")
-g = torch.cuda.CUDAGraph(); st = torch.cuda.Stream(); st.wait_stream(torch.cuda.current_stream())
-with torch.cuda.stream(st):
-    G.decode_attention(q, kcs[0], vcs[0], kvl, 0.088, out)
-    with torch.cuda.graph(g, stream=st):
-        for i in range(24): G.decode_attention(q, kcs[i % L], vcs[i % L], kvl, 0.088, out)
-torch.cuda.current_stream().wait_stream(st)
-us = timeit(lambda: g.replay()) / 24
-print(f"[unroll={os.environ.get('GROMA_DEC_UNROLL','4')}] decode_attention ctx=1030 in-graph: {us:.1f} us {2*B*H*1030*D*2/us/1e3:.0f} GB/s", flush=True)
+B = 16
+st = torch.cuda.Stream(); st.wait_stream(torch.cuda.current_stream())
 Hd = 4096
 for (N, K, S) in [(12288, 4096, 3), (22016, 4096, 6), (4096, 11008, 9)]:
     wl = [torch.randn(N, K, device="cuda").bfloat16() for _ in range(6)]
